@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the B200 robust-PCA hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c4|c2|c3|c5]
+                    [--dump-outputs DIR]
 
 One "step" = one full `rpca` solve to the reference's tolerance (sqrt(eps)) on the workload:
     c4 (default, the configuration the metric is quoted on): 1 000 000 x 256 FP64, rank 10 + 5 % sparse,
@@ -63,6 +64,38 @@ def measured_peaks():
         except Exception:
             pass
     return {"hbm_gbs": 6650.0}, "fallback"
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+DUMP_SEED = 20240
+
+
+def dump_outputs(path, rows, small):
+    """Write the outputs of one solve to `path`/<name>.npy as float64 so that two builds can be compared output for
+    output.  `rows`: arrays that share their first (row) dimension (torch tensors or NumPy arrays); when they do not
+    fit in DUMP_LIMIT_BYTES a fixed, seeded sample of rows is written, and `row_index.npy` names the rows.  `small`:
+    arrays written whole."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+
+    def host(v):
+        return np.asarray(v.cpu().numpy() if hasattr(v, "cpu") else v, dtype=np.float64)
+    out = {k: host(v) for k, v in small.items()}
+    m = next(iter(rows.values())).shape[0]
+    per_row = 8 * (1 + sum(math.prod(v.shape[1:]) for v in rows.values()))           # + 8 bytes of row_index
+    room = DUMP_LIMIT_BYTES - sum(a.nbytes for a in out.values()) - 128 * (len(out) + len(rows) + 1)   # npy headers
+    k = min(m, room // per_row)
+    idx = np.arange(m) if k == m else np.sort(np.random.default_rng(DUMP_SEED).choice(m, size=k, replace=False))
+    for name, v in rows.items():
+        if hasattr(v, "index_select"):                                 # torch: gather the sample on the device
+            import torch
+            v = v.index_select(0, torch.from_numpy(idx).to(v.device))
+        else:
+            v = v[idx]
+        out[name] = host(v)
+    out["row_index"] = idx.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -284,12 +317,16 @@ def run_b200(args, w, rank, world, local_rank):
         return float(t.item())
 
     parity = {}
+    last = {}                                                     # outputs of the last timed step (--dump-outputs)
     if w["kind"] == "rpca":
         D = T.synth.lowrank_sparse_cuda(r0, r1, N, dev, w["rank"], w["frac"], w["seed"], w["nonneg"])
         kw = dict(nonnegA=w["nonneg"], lam=lam)
 
-        def step():
+        def step(keep=False):
             A, E, s, sv, info = T.rpca(D, return_info=True, **kw)
+            if keep:
+                last["rows"] = {"A": A, "E": E, "U": s.U}
+                last["small"] = {"S": s.S, "Vt": s.Vt, "sv": sv, "iters": info["iters"]}
             return info["iters"]
 
         def parity_solve():
@@ -301,8 +338,10 @@ def run_b200(args, w, rank, world, local_rank):
     elif w["kind"] == "ga":
         X, q0 = T.synth.ga_data_cuda(r0, r1, N, dev, w["rank"], w["seed"])
 
-        def step():
+        def step(keep=False):
             Q, info = T.rpca_ga(X, w["rank"], q0=q0, return_info=True)
+            if keep:
+                last["rows"], last["small"] = {"Q": Q}, {"iters": info["iters"]}
             return sum(info["iters"])
 
         def parity_solve():
@@ -316,9 +355,11 @@ def run_b200(args, w, rank, world, local_rank):
         m = M                                                     # every rank holds the (small) signal
         lrf_last = {}
 
-        def step():
+        def step(keep=False):
             yf, info = T.lowrankfilter(yn, N, return_info=True)
             lrf_last["yf"], lrf_last["info"] = yf, info
+            if keep:
+                last["rows"], last["small"] = {"yf": yf}, {"iters": info["iters"], "sv": info["sv"]}
             return info["iters"]
 
         def parity_solve():
@@ -340,8 +381,8 @@ def run_b200(args, w, rank, world, local_rank):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     iters_total = 0
-    for _ in range(args.steps):
-        iters_total += step()
+    for i in range(args.steps):
+        iters_total += step(keep=args.dump_outputs is not None and i == args.steps - 1)
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
@@ -351,6 +392,8 @@ def run_b200(args, w, rank, world, local_rank):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms.item())
     value = iters_total / (ms * 1e-3)
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, last.pop("rows"), last.pop("small"))
 
     # ---- one profiled solve: per-phase device times for the roofline; one more for the cross-N parity digest ---
     T.set_profiling(True, local_rank)
@@ -556,7 +599,13 @@ def main():
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
     ap.add_argument("--rows", type=int, default=0, help="override the row count (debugging)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy "
+                    "(float64, at most 64 MB: a fixed, seeded row sample of the large outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl b200 in a single process")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = max(args.warmup, 1)
     w = dict(WORKLOADS[args.workload])

@@ -20,6 +20,7 @@ sys.path.insert(0, ROOT)
 import tls_oracle as O  # noqa: E402
 import tlsq_b200 as T  # noqa: E402
 
+STRIDE = 74                 # stored rows of the 3000 x 1000 case; column sums and norms pin the rows in between
 
 def main():
     warnings.simplefilter("ignore")
@@ -27,8 +28,10 @@ def main():
     t0 = time.time()
     D = T.synth.lowrank_sparse_np(3000, 1000, 8, 0.05, seed=21)
     r = O.rpca(D, iters=4, tol=0.0)
-    out["r1000_A_rows"] = np.ascontiguousarray(r.A[::37])
-    out["r1000_E_rows"] = np.ascontiguousarray(r.E[::37])
+    out["r1000_stride"] = STRIDE
+    out["r1000_A_rows"] = np.ascontiguousarray(r.A[::STRIDE])
+    out["r1000_E_rows"] = np.ascontiguousarray(r.E[::STRIDE])
+    out["r1000_A_colsum"], out["r1000_E_colsum"] = r.A.sum(axis=0), r.E.sum(axis=0)
     out["r1000_A_fro"], out["r1000_E_fro"] = np.linalg.norm(r.A), np.linalg.norm(r.E)
     out["r1000_S"], out["r1000_hist"] = r.s.S, r.hist
     print(f"rpca 3000x1000: {time.time() - t0:.0f} s", flush=True)

@@ -27,7 +27,7 @@ sys.path.insert(0, ROOT)
 import tls_oracle as O  # noqa: E402
 import tlsq_b200 as T  # noqa: E402  (only the NumPy generators in synth.py are used)
 
-STRIDE = 499
+STRIDE = 1497               # keeps the committed file under 1 MB; the digests pin the rows in between
 
 
 def reduce_rpca(out, name, r, D):
