@@ -100,10 +100,10 @@ def test_golden_vectors():
 ])
 def test_rpca_parity_fixed_iterations(M, N, r, kw, its, monkeypatch):
     D = T.synth.lowrank_sparse_np(M, N, r, 0.05, seed=M + N, nonneg=bool(kw.get("nonnegA")))
-    # n = 256: two-kernel pipeline (TMA-staged and register-prefetch streaming kernels) and the one-pass kernel
+    # n = 256: two-kernel pipeline and the one-pass kernel
     pipelines = [{}]
     if N == 256 and M >= 4096:
-        pipelines = [{"TLSQ_FUSED": "0"}, {"TLSQ_FUSED": "1"}, {"TLSQ_FUSED": "0", "TLSQ_STREAM_TMA": "0"}]
+        pipelines = [{"TLSQ_FUSED": "0"}, {"TLSQ_FUSED": "1"}]
     ref = None
     for env in pipelines:
         for k_, v_ in env.items():

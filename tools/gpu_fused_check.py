@@ -1,5 +1,5 @@
 """Debug driver for the fused one-pass ALM kernel (run on the GPU box): parity against the oracle + against the
-two-kernel pipeline (TLSQ_NO_FUSED=1), a few shapes, verbose numbers."""
+two-kernel pipeline (TLSQ_FUSED=0), a few shapes, verbose numbers."""
 import os, sys, time, warnings
 sys.path.insert(0, '.'); sys.path.insert(0, 'oracle')
 import numpy as np

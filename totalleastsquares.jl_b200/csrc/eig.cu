@@ -735,7 +735,7 @@ cudaError_t launch_eigh(const double* G, int n, const double* V0, EigWork w, dou
         else e = launch_cluster<8>(X0, V0, n, C, spc, tol, max_sweeps, w.Xo, w.Vo, w.info, run_flag, st);
         if (e != cudaSuccess) return e;
         if (launches) *launches += 1;
-    } else if (n <= 512 && getenv("TLSQ_JACOBI_GLOBAL") == nullptr) {
+    } else if (n <= 512) {
         // cooperative block tournament: C CTAs x 2 half-blocks of spc columns, C * 2 * spc >= n, spc <= 8
         const int mneed = (n + 1) / 2;
         int C = 16;

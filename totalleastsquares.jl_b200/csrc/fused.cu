@@ -526,7 +526,6 @@ size_t fused_partial_doubles(int sm_count) {
 }
 
 bool fused_eligible(const MatSrc& D, bool hankel, int64_t M, int64_t N) {
-    if (getenv("TLSQ_NO_FUSED") != nullptr) return false;      // test / comparison hook
     if (N != FN || M < 4096 || M >= ((int64_t)1 << 31)) return false;
     if (hankel) { if (D.ld != 1) return false; }        // Y / T live in padded (even) leading dimensions: any M
     else if ((M & 1) || (D.ld & 1) || (reinterpret_cast<uintptr_t>(D.p) & 15)) return false;

@@ -509,8 +509,6 @@ size_t ga_partial_doubles(int sm_count) { return (size_t)sm_count * GA_PSTRIDE; 
 
 namespace {
 bool ga_tma_ok(const double* X, int64_t d, int64_t N, int64_t ld, const double* part) {
-    const char* env = getenv("TLSQ_GA_TMA");
-    if (env && atoi(env) == 0) return false;
     return part && N <= GA_NC && N >= 8 && d >= 8192 && !(ld & 1) && !(reinterpret_cast<uintptr_t>(X) & 15) &&
            d < ((int64_t)1 << 31) && ga_encode_fn() != nullptr;
 }

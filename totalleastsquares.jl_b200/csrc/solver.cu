@@ -287,7 +287,6 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
     // Factored iterate: the low-rank iterate is kept as A_k = clamp(T_k V_k') (T: M x 32, V: N x 32).  The dense A is
     // then neither read nor written inside the loop; it is materialised only for the outputs, or for good (one-way
     // switch to the dense representation) if the rank estimate ever exceeds 32.
-    static const bool no_fact = getenv("TLSQ_NO_FACTORED") != nullptr;
     // Pipeline choice: the one-pass kernel needs S (Y in place) .. 2 S of device memory, the two-kernel pipeline up to
     // 4 S (Y x 2, W, Z); on B200 the two-kernel pipeline is currently the faster one when it fits (profiles/), so the
     // one-pass kernel is taken when memory asks for it, when the two-kernel pipeline is not available (odd row count
@@ -308,7 +307,7 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
     };
     const size_t free_b = device_free_bytes();
     const size_t ws_bytes = (size_t)4 << 30;
-    bool can_fused = !no_fact && !hk && fused_eligible(D, hankel, M, N);
+    bool can_fused = !hk && fused_eligible(D, hankel, M, N);
     if (can_fused && !syrk_ok && (o.A || o.E || o.U || o.S || o.Vt)) can_fused = false;   // padded leading dimension: factored outputs only
     // large embeddings (n > 512): always the two-kernel pipeline on a materialised W (column-chunked streaming epilogue,
     // T = W V_r by GEMM); the Gram takes the TMA SYRK when the shape allows it, else the generic DMMA kernel on W
@@ -339,7 +338,7 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
     bool use_w = pc.use_w;
     // the one-pass kernel moves Y / T tiles with TMA (16-byte strides): an odd row count gets a padded leading dimension
     const int64_t ldp = fused ? M + (M & 1) : M;
-    bool fact = (use_w || fused) && (!no_fact || large_n);
+    bool fact = use_w || fused;
     DevBuf bMean;
     double* meanbuf = nullptr;
     if (hk) { CK(bMean.alloc((size_t)(M + N) * 8, st)); meanbuf = bMean.as<double>(); }
@@ -441,8 +440,7 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
     }
     double* hp = h->h_pin;
     // fast eigen path state (dominant-subspace iteration, see eig_fast.cu)
-    static const bool no_fast = getenv("TLSQ_NO_FAST_EIG") != nullptr;
-    const bool fast_ok = eig_fast_supported(n) && !no_fast;
+    const bool fast_ok = eig_fast_supported(n);
     DevBuf bFast;
     EigFastWork fw = {};
     if (fast_ok) {
@@ -535,7 +533,6 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
     //  * while the host waits for ||Z||_F^2 of iteration k, the Gram and the eigen step of iteration k+1 are already
     //    enqueued ("run-ahead"; skipped when iteration k may converge, so at most nothing is wasted in practice).
     const bool no_ahead = getenv("TLSQ_NO_RUNAHEAD") != nullptr;
-    const bool no_spec = getenv("TLSQ_NO_SPECULATE") != nullptr;
     const bool trace = getenv("TLSQ_TRACE") != nullptr;
     auto now_us = []() {
         struct timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts);
@@ -601,7 +598,7 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
         // rank seen) and let the kernels check it; first iteration and the one-pass pipeline: fetch svp (short host sync).
         bool svp_known = false;
         int svp_guess = svp_pred > svp_last ? svp_pred : svp_last;
-        const bool speculate = use_w && !no_spec && k > 1;
+        const bool speculate = use_w && k > 1;
         if ((use_w || fused) && !speculate) {
             CK(cudaMemcpyAsync(hp + 1, dsvp, 4, cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
@@ -965,23 +962,18 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
         //   C'C = R'R                     Gram formed FROM THE DATA in the rotated, scaled basis + Cholesky
         //   K = R diag(s~) = U_K S V_K'   one-sided Jacobi of the n x n factor: K'K = V' W'W V exactly (to eps kappa(C)^2)
         //   W = (W V V_K S^-1) S (V V_K)' singular values to eps*s_1 like LAPACK's, V = V V_K, U = W V S^-1
-        const bool no_refine = getenv("TLSQ_NO_SVD_REFINE") != nullptr;
-        double* Vfin = Vs;
-        if (!no_refine) {
-            double* Cbuf = o.U;
-            if (!Cbuf) { if (!Zbuf) { CK(bZ.alloc(mn * 8, st)); Zbuf = bZ.as<double>(); } Cbuf = Zbuf; }
-            double* sc = lam2;                       // clamped scales s~
-            double* Gn2 = Gb[gi ^ 1];                // free n x n scratch
-            CK(launch_scale_cols_floor(Vs, sigma, n, 1.0e-8, sqA, sc, st, L));
-            CK(launch_gemm_any(Wfin, M, n, M, sqA, n, Cbuf, st, L));
-            CKR(gram_dense(h, Cbuf, M, n, G2));
-            CKR(allreduce(h, G2, (size_t)n * n, kNcclSum));
-            CK(launch_chol_upper(G2, n, st, L));
-            CK(launch_scale_cols_mul(G2, sc, n, sqB, st, L));
-            CK(launch_eigh(sqB, n, nullptr, ew, sigma, Vs2, sms, st, L, nullptr, 1));
-            CK(launch_gemm_nn(Vs, Vs2, n, Gn2, st, L));
-            Vfin = Gn2;
-        }
+        double* Cbuf = o.U;
+        if (!Cbuf) { if (!Zbuf) { CK(bZ.alloc(mn * 8, st)); Zbuf = bZ.as<double>(); } Cbuf = Zbuf; }
+        double* sc = lam2;                       // clamped scales s~
+        double* Vfin = Gb[gi ^ 1];               // refined basis V V_K (free n x n scratch)
+        CK(launch_scale_cols_floor(Vs, sigma, n, 1.0e-8, sqA, sc, st, L));
+        CK(launch_gemm_any(Wfin, M, n, M, sqA, n, Cbuf, st, L));
+        CKR(gram_dense(h, Cbuf, M, n, G2));
+        CKR(allreduce(h, G2, (size_t)n * n, kNcclSum));
+        CK(launch_chol_upper(G2, n, st, L));
+        CK(launch_scale_cols_mul(G2, sc, n, sqB, st, L));
+        CK(launch_eigh(sqB, n, nullptr, ew, sigma, Vs2, sms, st, L, nullptr, 1));
+        CK(launch_gemm_nn(Vs, Vs2, n, Vfin, st, L));
         if (o.S) CK(cudaMemcpyAsync(o.S, sigma, (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
         if (o.Vt) CK(launch_transpose(Vfin, N, N, o.Vt, st, L));
         if (o.U) {
@@ -1105,7 +1097,6 @@ int rpca_ga_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r
     double* part = bPart.as<double>();
     double* hp = h->h_pin;
     const bool no_ahead = getenv("TLSQ_NO_RUNAHEAD") != nullptr;
-    const bool no_fuse = getenv("TLSQ_GA_NO_FUSE") != nullptr;
     CK(cudaMemcpyAsync(Xw, X, dn * 8, cudaMemcpyDeviceToDevice, st));                    // X = copy(X)   :257
 
     // q = randn(d); q ./= norm(q)   (:286-287) -- the draw comes from the caller
@@ -1184,24 +1175,20 @@ int rpca_ga_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r
         CK(cudaMemcpyAsync(Q + i * d, q, (size_t)d * 8, cudaMemcpyDeviceToDevice, st));  // :269
         if (i + 1 == r) break;                          // X is a private copy: deflating after the last component is moot
         // Xs1 = q'X (:271) = (X'mu) / ||mu|| -- already known from the last sweep, no extra pass over X
-        bool fused_done = false;
-        if (!no_fuse) {
-            CK(launch_ga_xs(tl, N, xs, st, L));
-            CKR(normalise_start(i + 1, qnext));
-            CK(cudaMemsetAsync(n2, 0, (size_t)N * 8, st));
-            CK(cudaMemsetAsync(tb[0], 0, (size_t)(N + 1) * 8, st));
-            // X -= q Xs1 (:272) fused with the norms (:265) and first dot products (:292) of the next component
-            cudaError_t fe = launch_ga_deflate_fused(Xw, d, N, d, q, xs, qnext, n2, tb[0], part, sms, st, L);
-            if (fe == cudaSuccess) {
-                CKR(allreduce(h, n2, (size_t)N, kNcclSum));
-                CKR(allreduce(h, tb[0], (size_t)N, kNcclSum));
-                fused_done = true;
-                head_ready = true;
-            } else if (fe != cudaErrorNotSupported) {
-                CK(fe);
-            }
-        }
-        if (!fused_done) {
+        CK(launch_ga_xs(tl, N, xs, st, L));
+        CKR(normalise_start(i + 1, qnext));
+        CK(cudaMemsetAsync(n2, 0, (size_t)N * 8, st));
+        CK(cudaMemsetAsync(tb[0], 0, (size_t)(N + 1) * 8, st));
+        // X -= q Xs1 (:272) fused with the norms (:265) and first dot products (:292) of the next component
+        cudaError_t fe = launch_ga_deflate_fused(Xw, d, N, d, q, xs, qnext, n2, tb[0], part, sms, st, L);
+        if (fe == cudaSuccess) {
+            CKR(allreduce(h, n2, (size_t)N, kNcclSum));
+            CKR(allreduce(h, tb[0], (size_t)N, kNcclSum));
+            head_ready = true;
+        } else if (fe != cudaErrorNotSupported) {
+            CK(fe);
+        } else {
+            // the shape does not take the TMA sweep: Xs1 and the deflation as separate passes
             CK(cudaMemsetAsync(xs, 0, (size_t)N * 8, st));
             CK(launch_ga_sweep(GA_DOTS, Xw, d, N, d, q, nullptr, nullptr, xs, sms, st, L, part));  // Xs1 = q'X   :271
             CKR(allreduce(h, xs, (size_t)N, kNcclSum));
@@ -1228,7 +1215,6 @@ int lowrankfilter_dev(tlsq_handle* h, const double* y, int64_t Ns, int64_t n, in
     // Factored unhankel (lag 1, tall enough for the factored iterate): A is never materialised -- the anti-diagonal
     // sums are taken straight from A_k = clamp(T_k V_k'); sharded runs all-reduce the Ns partial sums.
     {
-        static const bool no_fact = getenv("TLSQ_NO_FACTORED") != nullptr;
         int64_t r0, Kl, per, Klast, r0last;
         shard_hankel_rows(K, h->nranks, h->rank, &r0, &Kl);
         shard_hankel_rows(K, h->nranks, 0, &r0last, &per);
@@ -1238,7 +1224,7 @@ int lowrankfilter_dev(tlsq_handle* h, const double* y, int64_t Ns, int64_t n, in
             return rows >= 1 && (syrk_tma_eligible(reinterpret_cast<const double*>(uintptr_t(256)), rows, n, rows) ||
                                  fused_eligible(MatSrc{y, 1}, true, rows, n));
         };
-        if (lag == 1 && !no_fact && K >= n && n <= kEigMaxN && (h->nranks == 1 || shard_ok(per)) && shard_ok(Klast)) {
+        if (lag == 1 && K >= n && n <= kEigMaxN && (h->nranks == 1 || shard_ok(per)) && shard_ok(Klast)) {
             CKR(check_rpca_args(Kl, n, p));
             DevBuf bSum;
             CK(bSum.alloc((size_t)Ns * 8, st));

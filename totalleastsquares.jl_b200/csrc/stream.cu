@@ -33,10 +33,11 @@ __device__ __forceinline__ double dot_rp(const double (&t)[RP > 0 ? RP : 1], con
 }
 
 // PH: 0 = both loops in one kernel; 1 = only T = (W V_r) .* f (written to a.Tn); 2 = only the element-wise pass (T_k read
-// back from a.Tn).  The split form (1 then 2, FACT only) runs each loop at a higher occupancy.
+// back from a.Tn).  FACT at a rank above 0 always runs the split form (1 then 2): each loop at a higher occupancy.
 template <int RP, bool HANKEL, bool FACT, int PH>
 __global__ void __launch_bounds__(128)
 alm_stream_kernel(const EpiArgs a, const double* __restrict__ W, int svp_host, const int* __restrict__ svp_dev) {
+    static_assert(!(FACT && PH == 0 && RP > 0), "FACT at a rank above 0 runs the split form (T_{k-1} is loaded by PH 2)");
     // Rank of this iteration: either known on the host, or (speculative launch, solver.cu) read from the device scalar
     // the eigen step just wrote.  The launch was specialised on a GUESS of the rank; if the actual rank does not fit
     // the guess the whole grid returns before touching anything and the host relaunches with the right RP.
@@ -57,10 +58,7 @@ alm_stream_kernel(const EpiArgs a, const double* __restrict__ W, int svp_host, c
     }
     __syncthreads();
     double zz = 0.0;
-#ifndef TLSQ_STREAM_UB
-#define TLSQ_STREAM_UB 4
-#endif
-    constexpr int UB = TLSQ_STREAM_UB;         // columns whose loads are issued together
+    constexpr int UB = 4;                      // columns whose loads are issued together
     for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < a.M;
          row += (int64_t)gridDim.x * blockDim.x) {
         // ---- T[row, :] = f .* (W[row, :] V_r): one streaming read of the materialised SVT input ----------------
@@ -105,10 +103,7 @@ alm_stream_kernel(const EpiArgs a, const double* __restrict__ W, int svp_host, c
             for (int c = 0; c < RP; ++c) tr[c] *= fsm[c];
             if (FACT) {
 #pragma unroll
-                for (int c = 0; c < RP; ++c) {
-                    if (PH == 0) tp[c] = c < a.svp_prev ? __ldg(a.Tp + (int64_t)c * a.M + row) : 0.0;
-                    a.Tn[(int64_t)c * a.M + row] = tr[c];
-                }
+                for (int c = 0; c < RP; ++c) a.Tn[(int64_t)c * a.M + row] = tr[c];
             }
         }
         if (PH == 1) continue;
@@ -250,8 +245,6 @@ template <int RP>
 cudaError_t launch_stream_rp(const EpiArgs& a, const double* W, int svp, const int* svp_dev, bool hankel, int sm_count,
                              cudaStream_t st) {
     const bool fact = a.Tn != nullptr;
-    static const bool split_env = getenv("TLSQ_STREAM_SPLIT") ? atoi(getenv("TLSQ_STREAM_SPLIT")) != 0 : true;
-    const bool split = fact && split_env && RP > 0;
     int64_t blocks = (a.M + 127) / 128;
     int64_t cap = (int64_t)sm_count * 16;
     if (blocks > cap) blocks = cap;
@@ -293,13 +286,13 @@ cudaError_t launch_stream_rp(const EpiArgs& a, const double* W, int svp, const i
         return cudaGetLastError();
     }
     const size_t sm1 = (size_t)a.N * RP * sizeof(double);
-    if (split) {
+    if (!fact) {
+        if (hankel) TLSQ_STREAM_LAUNCH(true, false, 0, sm1); else TLSQ_STREAM_LAUNCH(false, false, 0, sm1);
+    } else if constexpr (RP == 0) {
+        if (hankel) TLSQ_STREAM_LAUNCH(true, true, 0, 2 * sm1); else TLSQ_STREAM_LAUNCH(false, true, 0, 2 * sm1);
+    } else {
         if (hankel) { TLSQ_STREAM_LAUNCH(true, true, 1, sm1); if (e == cudaSuccess) TLSQ_STREAM_LAUNCH(true, true, 2, 2 * sm1); }
         else        { TLSQ_STREAM_LAUNCH(false, true, 1, sm1); if (e == cudaSuccess) TLSQ_STREAM_LAUNCH(false, true, 2, 2 * sm1); }
-    } else if (hankel) {
-        if (fact) TLSQ_STREAM_LAUNCH(true, true, 0, 2 * sm1); else TLSQ_STREAM_LAUNCH(true, false, 0, sm1);
-    } else {
-        if (fact) TLSQ_STREAM_LAUNCH(false, true, 0, 2 * sm1); else TLSQ_STREAM_LAUNCH(false, false, 0, sm1);
     }
 #undef TLSQ_STREAM_LAUNCH
     if (e != cudaSuccess) return e;

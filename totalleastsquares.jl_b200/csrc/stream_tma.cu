@@ -364,9 +364,7 @@ cudaError_t launch_rp(const EpiArgs& a, const double* W, int svp, const int* svp
 // Can the TMA-staged pair replace the register-prefetch kernels for this launch?  (factored iterate, all columns in one
 // launch, 16-byte aligned bases and strides, both V blocks + the ring within shared memory)
 bool stream_tma_eligible(const EpiArgs& a, const double* W, int rp, bool hankel) {
-    const char* env = getenv("TLSQ_STREAM_TMA");       // read per call: tests toggle it
-    const bool off = env && atoi(env) == 0;
-    if (off || rp < 4 || rp > 12 || !a.Tn || !a.Tp || !a.Wn || a.c1 > 0) return false;   // rp > 12: > 128 registers at 512 threads
+    if (rp < 4 || rp > 12 || !a.Tn || !a.Tp || !a.Wn || a.c1 > 0) return false;   // rp > 12: > 128 registers at 512 threads
     if (a.M < 16384 || a.N < 8 || (a.N & 7) || (a.ldw & 1) || !aligned16(W) || !aligned16(a.Yp)) return false;
     if (!hankel && ((a.D.ld & 1) || !aligned16(a.D.p))) return false;
     if (a.M >= (int64_t)1 << 31) return false;
