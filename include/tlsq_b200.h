@@ -153,8 +153,9 @@ int tlsq_rpca_ga_f64_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, 
                          double tol, int64_t iters, double* Q, int64_t* iters_done);
 
 /* rpca_ga with the reference's pluggable robust averages (keyword mu, :255,294): mu_kind 0 = mu! (:308-316),
- * 1 = entrywise_trimmed_mean(s, w, U, P = mu_p) (:323-333), 2 = entrywise_median (:349-357).  A per-row sort over the N
- * observations (N <= 16384; beyond 1024 a slower one-row-per-CTA sort).  Rows may be sharded like tlsq_rpca_ga_f64.   */
+ * 1 = entrywise_trimmed_mean(s, w, U, P = mu_p) (:323-333), 2 = entrywise_median (:349-357), for any number N of
+ * observations: a per-row sort up to 16384 observations, per-row radix selection over streaming sweeps of X beyond.
+ * Rows may be sharded like tlsq_rpca_ga_f64.                                                                        */
 int tlsq_rpca_ga_mu_f64(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r, const double* q0,
                         double tol, int64_t iters, int mu_kind, double mu_p, double* Q, int64_t* iters_done);
 int tlsq_rpca_ga_mu_f64_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r, const double* q0,
@@ -200,6 +201,11 @@ int tlsq_plan_fused_strips(uint8_t* tile_row, uint8_t* strip_col);
 int tlsq_gram_f64_dev(tlsq_handle* h, const double* X, int64_t M, int64_t n, double* G);
 /* eigen-decomposition of a symmetric PSD n x n matrix (one-sided Jacobi): lam sorted descending, V columns     */
 int tlsq_eigh_f64_dev(tlsq_handle* h, const double* G, int64_t n, double* lam, double* V);
+/* s (length d) = the reference's robust average mu(s, w, U) of U (d x N, column-major) with weights w (length N):
+ * kind 1 = entrywise_trimmed_mean with fraction P (:323-333), kind 2 = entrywise_median (:349-357; for N = 1 the
+ * single entry).  Always takes the per-row radix selection kernels that rpca_ga uses beyond 16384 observations.     */
+int tlsq_robust_average_f64_dev(tlsq_handle* h, const double* U, int64_t d, int64_t N, const double* w, int kind,
+                                double P, double* s);
 
 #ifdef __cplusplus
 }

@@ -27,7 +27,7 @@ from ._cabi import TlsqError, load  # noqa: F401
 
 __all__ = ["rpca", "rpca_ga", "lowrankfilter", "hankel", "unhankel", "rtls", "tls", "entrywise_trimmed_mean",
            "entrywise_median", "mu_mean", "SVD", "TlsqError", "get_handle",
-           "init_distributed", "launch_count", "gram", "eigh", "set_profiling", "get_profile", "PHASES"]
+           "init_distributed", "launch_count", "gram", "eigh", "robust_average", "set_profiling", "get_profile", "PHASES"]
 
 
 class SVD(NamedTuple):
@@ -630,3 +630,25 @@ def eigh(G):
     _cabi.check(load().tlsq_eigh_f64_dev(_handle_for(Ga), Ga.ptr, n, C.c_void_p(lam.data_ptr()),
                                          C.c_void_p(Vc.data_ptr())))
     return lam, Vc.t()
+
+
+def robust_average(U, w, mu=entrywise_trimmed_mean, P: float = 0.1):
+    """s = mu(s, w, U) for ``mu = entrywise_trimmed_mean`` (fraction ``P``, src/robustPCA.jl:323-333) or
+    ``entrywise_median`` (:349-357) through the per-row selection kernels (U: d x N and w: N, CUDA float64 tensors)."""
+    import torch
+    Ua, wa = _Arr(U, "U"), _Arr(w, "w")
+    if not (Ua.torch and wa.torch):
+        raise TypeError("robust_average: pass CUDA tensors")
+    if len(Ua.shape) != 2 or tuple(wa.shape) != (Ua.shape[1],):
+        raise ValueError("robust_average: U must be d x N and w of length N")
+    if mu is entrywise_trimmed_mean:
+        kind = 1
+    elif mu is entrywise_median:
+        kind = 2
+    else:
+        raise NotImplementedError("robust_average: mu must be entrywise_trimmed_mean or entrywise_median")
+    d, N = Ua.shape
+    s = torch.empty((d,), dtype=torch.float64, device=Ua.obj.device)
+    _cabi.check(load().tlsq_robust_average_f64_dev(_handle_for(Ua), Ua.ptr, d, N, wa.ptr, kind, float(P),
+                                                   C.c_void_p(s.data_ptr())))
+    return s

@@ -65,6 +65,7 @@ SIGNATURES = {
     "tlsq_plan_hankel_shard": (C.c_int, [C.c_int64, C.c_int, C.c_int, c_i64p, c_i64p]),
     "tlsq_gram_f64_dev": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp]),
     "tlsq_eigh_f64_dev": (C.c_int, [vp, vp, C.c_int64, vp, vp]),
+    "tlsq_robust_average_f64_dev": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp, C.c_int, C.c_double, vp]),
 }
 
 

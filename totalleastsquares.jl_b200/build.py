@@ -16,7 +16,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtlsq_b200.so")
-SOURCES = ["gram.cu", "syrk_tma.cu", "eig.cu", "eig_fast.cu", "epilogue.cu", "stream.cu", "stream_tma.cu", "fused.cu", "gemm.cu", "elementwise.cu", "ga.cu", "solver.cu"]
+SOURCES = ["gram.cu", "syrk_tma.cu", "eig.cu", "eig_fast.cu", "epilogue.cu", "stream.cu", "stream_tma.cu", "fused.cu", "gemm.cu", "elementwise.cu", "ga.cu", "ga_select.cu", "solver.cu"]
 HEADERS = ["common.cuh", "kernels.h", os.path.join("..", "..", "include", "tlsq_b200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -322,10 +322,24 @@ cudaError_t launch_ga_deflate_fused(double* X, int64_t d, int64_t N, int64_t ld,
 cudaError_t launch_ga_xs(const double* t, int64_t N, double* xs, cudaStream_t st, int64_t* launches);
 // robust entry-wise averages (:323-333, :349-357): out[j] (length d) from a per-row sort over the N observations;
 // kind 1 = trimmed mean (fraction P dropped on each side), 2 = median.  N <= 1024: 8 / 32 rows per tile, one warp per
-// row; up to kGaRobustMaxN observations: one CTA per row (slow path).
+// row; up to kGaRobustMaxN observations: one CTA per row.  Longer rows take the selection kernels below.
 constexpr int kGaRobustMaxN = 16384;
 cudaError_t launch_ga_robust(const double* X, int64_t d, int64_t N, int64_t ld, const double* sgn, const double* n2,
                              int kind, double P, double* out, int sm_count, cudaStream_t st, int64_t* launches);
+// The same averages for any N (ga_select.cu): per-row radix selection over streaming sweeps of X, same order as
+// launch_ga_robust (ascending key, then column; -0.0 == +0.0; NaN keys last).  Keys u = X[j,n] / sqrt(n2[n]) and
+// weights w_n = wt[n] sqrt(n2[n]); with n2 == nullptr X holds U itself and wt the weights.  ws: ga_select_bytes().
+//   kind 2: out = the median average (:349-357).
+//   kind 1: the two boundaries of every row's kept range [floor(P N), floor((1-P) N)) into ws; they depend on X and n2
+//           only, so they hold for a whole component.  launch_ga_trimmed_sweep then gives out = the trimmed mean with
+//           the current weights (:323-333), summed in a fixed order.
+size_t ga_select_bytes(int64_t d, int64_t N, int sm_count);
+cudaError_t launch_ga_select(const double* X, int64_t d, int64_t N, int64_t ld, const double* wt, const double* n2,
+                             int kind, double P, void* ws, double* out, int sm_count, cudaStream_t st,
+                             int64_t* launches);
+cudaError_t launch_ga_trimmed_sweep(const double* X, int64_t d, int64_t N, int64_t ld, const double* wt,
+                                    const double* n2, double P, const void* ws, double* out, int sm_count,
+                                    cudaStream_t st, int64_t* launches);
 // s[n] = sign(t[n]) (0 if norms[n]==0), sumw = sum_n s[n]*norms[n]            (:292, :310-312)
 cudaError_t launch_ga_signs(const double* t, const double* norms2, int64_t N, double* s, double* sumw,
                             cudaStream_t st, int64_t* launches);

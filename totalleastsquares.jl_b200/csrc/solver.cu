@@ -1088,6 +1088,11 @@ int rpca_ga_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r
     CK(bQn.alloc((size_t)d * 8, st));
     CK(bMu.alloc((size_t)d * 8, st)); CK(bXs.alloc((size_t)N * 8, st)); CK(bSc.alloc(8 * 8, st));
     CK(bPart.alloc(ga_partial_doubles(sms) * 8, st));
+    // robust averages over more than kGaRobustMaxN observations: per-row selection (ga_select.cu) instead of a sort
+    const bool select = mu_kind != 0 && N > kGaRobustMaxN;
+    DevBuf bSel;
+    if (select) CK(bSel.alloc(ga_select_bytes(d, N, sms), st));
+    void* sel = bSel.p;
     double* Xw = bX.as<double>(); double* n2 = bN2.as<double>();
     double* tb[2] = {bT.as<double>(), bT2.as<double>()};           // dot products: iteration `it` writes tb[it & 1]
     double* s = bS.as<double>(); double* mu = bMu.as<double>();
@@ -1122,6 +1127,8 @@ int rpca_ga_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r
             CK(cudaMemcpyAsync(qb[0], qnext, (size_t)d * 8, cudaMemcpyDeviceToDevice, st));
         }
         head_ready = false;
+        // trimmed mean: the keys X[j,n] / ||x_n|| are fixed until the deflation, so are the rows' kept ranges
+        if (select && mu_kind == 1) CK(launch_ga_select(Xw, d, N, d, s, n2, 1, mu_p, sel, nullptr, sms, st, L));
         // One Grassmann iteration on the device (:291-296): signs from the dot products of the previous sweep (tb[(it-1)&1]),
         // one sweep (mu, next dot products into tb[it&1], ||mu||^2), q_new into the OTHER q buffer, ||q_new - q||^2
         // into slot `it & 1`.
@@ -1138,7 +1145,9 @@ int rpca_ga_dev(tlsq_handle* h, const double* X, int64_t d, int64_t N, int64_t r
                 // to a shard), then ||mu||^2 and the dot products of the NEXT iteration with q = mu/||mu|| -- the sign
                 // of u_n'q equals the sign of x_n'mu, so the dots are taken with mu directly
                 Phase ph(h, TLSQ_PHASE_GA_SWEEP);
-                CK(launch_ga_robust(Xw, d, N, d, s, n2, mu_kind, mu_p, mu, sms, st, L));
+                if (!select) CK(launch_ga_robust(Xw, d, N, d, s, n2, mu_kind, mu_p, mu, sms, st, L));
+                else if (mu_kind == 1) CK(launch_ga_trimmed_sweep(Xw, d, N, d, s, n2, mu_p, sel, mu, sms, st, L));
+                else CK(launch_ga_select(Xw, d, N, d, s, n2, 2, mu_p, sel, mu, sms, st, L));
                 CK(launch_vec_sumsq(mu, d, t + N, sms, st, L));
                 CK(launch_ga_sweep(GA_DOTS, Xw, d, N, d, mu, nullptr, nullptr, t, sms, st, L, part));
             }
@@ -1886,7 +1895,6 @@ int tlsq_rpca_ga_mu_f64_dev(tlsq_handle* h, const double* X, int64_t d, int64_t 
                             double tol, int64_t iters, int mu_kind, double mu_p, double* Q, int64_t* iters_done) {
     CKR(use_device(h));
     if (mu_kind < 0 || mu_kind > 2) return set_err(TLSQ_ERR_ARG, "rpca_ga: mu_kind must be 0 (mean), 1 (trimmed mean) or 2 (median)");
-    if (mu_kind && N > kGaRobustMaxN) return set_err(TLSQ_ERR_UNSUPPORTED, "rpca_ga: robust averages support at most %d observations", kGaRobustMaxN);
     if (mu_kind == 2 && N < 2) return set_err(TLSQ_ERR_ARG, "rpca_ga: entrywise_median needs at least 2 observations (I[end / 2], src/robustPCA.jl:353)");
     return rpca_ga_dev(h, X, d, N, r, q0, tol, iters, Q, iters_done, mu_kind, mu_p);
 }
@@ -1896,7 +1904,6 @@ int tlsq_rpca_ga_mu_f64(tlsq_handle* h, const double* X, int64_t d, int64_t N, i
     CKR(use_device(h));
     if (!X || !q0 || !Q || d < 1 || N < 1 || r < 1) return set_err(TLSQ_ERR_ARG, "rpca_ga: bad arguments");
     if (mu_kind < 0 || mu_kind > 2) return set_err(TLSQ_ERR_ARG, "rpca_ga: mu_kind must be 0 (mean), 1 (trimmed mean) or 2 (median)");
-    if (mu_kind && N > kGaRobustMaxN) return set_err(TLSQ_ERR_UNSUPPORTED, "rpca_ga: robust averages support at most %d observations", kGaRobustMaxN);
     if (mu_kind == 2 && N < 2) return set_err(TLSQ_ERR_ARG, "rpca_ga: entrywise_median needs at least 2 observations (I[end / 2], src/robustPCA.jl:353)");
     cudaStream_t st = h->stream;
     DevBuf bX, bq0, bQ;
@@ -2059,6 +2066,29 @@ int tlsq_eigh_f64_dev(tlsq_handle* h, const double* G, int64_t n, double* lam, d
     ew.perm = reinterpret_cast<int*>(base); base += n;
     ew.info = reinterpret_cast<int*>(base);
     CK(launch_eigh(G, (int)n, nullptr, ew, lam, V, h->sm_count, st, &h->launches));
+    CK(cudaStreamSynchronize(st));
+    return TLSQ_OK;
+}
+
+int tlsq_robust_average_f64_dev(tlsq_handle* h, const double* U, int64_t d, int64_t N, const double* w, int kind,
+                                double P, double* s) {
+    if (!h) {
+        int n = 0;
+        if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
+            cudaGetLastError();
+            return set_err(TLSQ_ERR_NO_DEVICE, "no CUDA device available (this library has no CPU fallback)");
+        }
+    }
+    CKR(use_device(h));
+    if (!U || !w || !s || d < 1 || N < 1) return set_err(TLSQ_ERR_ARG, "robust_average: bad arguments");
+    if (kind != 1 && kind != 2) return set_err(TLSQ_ERR_ARG, "robust_average: kind must be 1 (trimmed mean) or 2 (median)");
+    if (kind == 1 && !(P >= 0.0 && P <= 1.0)) return set_err(TLSQ_ERR_ARG, "robust_average: P must lie in [0, 1]");
+    if (N > (int64_t)0xffffffffLL) return set_err(TLSQ_ERR_UNSUPPORTED, "robust_average: more than 2^32 - 1 observations");
+    cudaStream_t st = h->stream;
+    DevBuf bW;
+    CK(bW.alloc(ga_select_bytes(d, N, h->sm_count), st));
+    CK(launch_ga_select(U, d, N, d, w, nullptr, kind, P, bW.p, s, h->sm_count, st, &h->launches));
+    if (kind == 1) CK(launch_ga_trimmed_sweep(U, d, N, d, w, nullptr, P, bW.p, s, h->sm_count, st, &h->launches));
     CK(cudaStreamSynchronize(st));
     return TLSQ_OK;
 }

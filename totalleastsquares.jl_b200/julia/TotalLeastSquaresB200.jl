@@ -160,7 +160,7 @@ end
     entrywise_trimmed_mean / entrywise_median
 
 Tags for the reference's robust averages (src/robustPCA.jl:323-333, :349-357) in `rpca_ga(...; μ = ...)`; the per-row
-sorts run on the GPU.  `μ = (entrywise_trimmed_mean, P)` selects a trimming fraction other than 0.1.
+sorts (per-row selection beyond 16 384 observations) run on the GPU, for any number of observations.  `μ = (entrywise_trimmed_mean, P)` selects a trimming fraction other than 0.1.
 """
 entrywise_trimmed_mean(args...) = error("pass it as rpca_ga(X, r; μ = entrywise_trimmed_mean)")
 entrywise_median(args...) = error("pass it as rpca_ga(X, r; μ = entrywise_median)")
