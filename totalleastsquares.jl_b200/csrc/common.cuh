@@ -61,6 +61,23 @@ __device__ __forceinline__ double warp_max(double v) {
 }
 
 // ---------------------------------------------------------------------------------------------------
+// Sort key of the robust Grassmann averages (the reference's sortperm over a row, Julia's isless): an order-preserving
+// map double -> uint64 with -0.0 == +0.0 and every NaN (a zero column's 0 / 0) above +inf.  Shared by the per-row
+// sorts (ga.cu) and the per-row selection (ga_select.cu), so both paths order a row identically.  No key maps above
+// ~0 (NaN), so padding slots that hold ~0 with an index >= N sort after every real element.
+// ---------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint64_t sel_order(double u) {
+    uint64_t b = (uint64_t)__double_as_longlong(u);
+    if ((b << 1) == 0) b = 0;                                              // -0.0 -> +0.0
+    if ((b & 0x7fffffffffffffffull) > 0x7ff0000000000000ull) return ~0ull;   // NaN: last (Julia's isless)
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+// the double a sel_order key came from (-0.0 comes back as +0.0, a NaN key as a NaN)
+__device__ __forceinline__ double sel_value(uint64_t k) {
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+
+// ---------------------------------------------------------------------------------------------------
 // Plane rotation that (nearly) annihilates gamma = x_p . x_q given alpha = |x_p|^2, beta = |x_q|^2.
 // The tangent only needs ~20 bits (a slightly inexact angle still converges; later sweeps finish the job), so it is
 // built from the single-instruction MUFU reciprocal / rsqrt approximations instead of four IEEE FP64 div/sqrt

@@ -444,12 +444,9 @@ cudaError_t launch_unhankel_factors(const double* T, int64_t ldt, const double* 
         if (launches) *launches += 1;
         return cudaGetLastError();
     }
-    static size_t attr = 0;
-    if (smem > attr) {
-        cudaError_t e = cudaFuncSetAttribute(unhankel_factors_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        attr = smem;
-    }
+    // function attributes are per device: set on every launch (a process may run on several GPUs)
+    cudaError_t e = cudaFuncSetAttribute(unhankel_factors_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
     int64_t blocks = (Ns + 255) / 256;
     if (blocks > (int64_t)sm_count * 4) blocks = (int64_t)sm_count * 4;
     unhankel_factors_kernel<<<(unsigned)blocks, 256, smem, st>>>(T, ldt, V, rp, nonnegA, r0, Kl, (int)n, Ns, sum);

@@ -358,7 +358,9 @@ inline int vec_grid(int64_t total, int sm_count) {
 // entrywise_median): per ROW j of the normalised data U[j,n] = X[j,n]/||x_n|| a sort over the N observations.
 // A block stages 32 consecutive rows x N columns in shared memory with coalesced loads (lanes along rows); every
 // warp then sorts its rows one after the other with a bitonic network on (key, index) pairs -- the index breaks ties
-// like the reference's stable sortperm.
+// like the reference's stable sortperm.  Keys are mapped by sel_order (common.cuh), the order of the selection path
+// above kGaRobustMaxN: -0.0 == +0.0 and NaN keys (zero columns, 0 / 0) last.  Padding slots [N, NP2) hold the largest
+// key and sort after the NaNs on their index, so the first N sorted slots are always real columns.
 //   kind 1: keys = U[j,:]; s[j] = sum_{n in I} w_n U[j,n] / sum_{n in I} w_n, I = sorted[lo:hi)
 //   kind 2: keys = w .* U[j,:]; m = sorted[N/2 - 1]; s[j] = sign(w_m) U[j,m]
 // w_n = sgn_n * sqrt(n2_n) (sgn from the previous sweep's dot products, :291-293).
@@ -371,16 +373,15 @@ ga_robust_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int RT
     const int TS = RT + 1;                                // RT rows per tile (32, or 8 for long observation axes)
     double* tile = smr;                                   // [N][RT + 1]  (padded: rows along the fast index)
     double* wv = tile + (size_t)N * TS;                   // [N] weights
-    double* inv = wv + N;                                 // [N] 1 / ||x_n||
-    double* keys = inv + N;                               // [8 warps][NP2]
+    double* nrm = wv + N;                                 // [N] ||x_n||
+    uint64_t* keys = reinterpret_cast<uint64_t*>(nrm + N);   // [8 warps][NP2]  sel_order keys
     int* idxs = reinterpret_cast<int*>(keys + 8 * NP2);   // [8 warps][NP2]
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int n = tid; n < N; n += 256) {
         const double nr = sqrt(n2[n]);
         wv[n] = sgn[n] * nr;
-        inv[n] = nr;
+        nrm[n] = nr;
     }
-    const double INF = __longlong_as_double(0x7ff0000000000000LL);
     for (int64_t r0 = (int64_t)blockIdx.x * RT; r0 < d; r0 += (int64_t)gridDim.x * RT) {
         __syncthreads();
         for (int idx = tid; idx < N * RT; idx += 256) {
@@ -389,18 +390,19 @@ ga_robust_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int RT
             tile[n * TS + r] = row < d ? __ldg(X + (int64_t)n * ld + row) : 0.0;
         }
         __syncthreads();
-        double* kk = keys + warp * NP2;
+        uint64_t* kk = keys + warp * NP2;
         int* ii = idxs + warp * NP2;
         for (int rr = warp; rr < RT; rr += 8) {
             const int64_t row = r0 + rr;
             if (row >= d) break;
             for (int n = lane; n < NP2; n += 32) {
-                double u = INF;
+                uint64_t key = ~0ull;                                           // padding: after NaN keys (index >= N)
                 if (n < N) {
-                    u = tile[n * TS + rr] / inv[n];                              // U[j,n] = X[j,n] / Xnorms[n]   :266
+                    double u = tile[n * TS + rr] / nrm[n];                       // U[j,n] = X[j,n] / Xnorms[n]   :266
                     if (kind == 2) u = wv[n] * u;
+                    key = sel_order(u);
                 }
-                kk[n] = u;
+                kk[n] = key;
                 ii[n] = n;
             }
             __syncwarp();
@@ -410,7 +412,7 @@ ga_robust_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int RT
                         const int a = 2 * t - (t & (j - 1));                      // lower index of the pair (bit j clear)
                         const int b = a + j;
                         const bool up = (a & k) == 0;
-                        const double ka = kk[a], kb = kk[b];
+                        const uint64_t ka = kk[a], kb = kk[b];
                         const int ia = ii[a], ib = ii[b];
                         const bool gt = (ka > kb) || (ka == kb && ia > ib);
                         if (gt == up) { kk[a] = kb; kk[b] = ka; ii[a] = ib; ii[b] = ia; }
@@ -420,8 +422,9 @@ ga_robust_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int RT
             if (kind == 1) {
                 double num = 0.0, den = 0.0;
                 for (int p = lo + lane; p < hi; p += 32) {
-                    const double w = wv[ii[p]];
-                    num = fma(w, kk[p], num);
+                    const int n = ii[p];
+                    const double w = wv[n];
+                    num = fma(w, sel_value(kk[p]), num);                           // w_n U[j,n]
                     den += w;
                 }
                 num = warp_sum(num);
@@ -430,7 +433,7 @@ ga_robust_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int RT
             } else if (lane == 0) {
                 const int m = ii[N / 2 - 1];
                 const double w = wv[m];
-                const double u = tile[m * TS + rr] / inv[m];
+                const double u = tile[m * TS + rr] / nrm[m];
                 out[row] = (w > 0.0 ? 1.0 : (w < 0.0 ? -1.0 : 0.0)) * u;
             }
             __syncwarp();
@@ -444,22 +447,22 @@ ga_robust_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int RT
 __global__ void __launch_bounds__(512)
 ga_robust_big_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, int64_t ld, const double* __restrict__ sgn,
                      const double* __restrict__ n2, int kind, int lo, int hi, double* __restrict__ out) {
-    extern __shared__ double smb[];
-    double* kk = smb;                                     // [NP2]
+    extern __shared__ uint64_t smb[];
+    uint64_t* kk = smb;                                   // [NP2]  sel_order keys
     int* ii = reinterpret_cast<int*>(kk + NP2);           // [NP2]
     __shared__ double rn[16], rd[16];
     const int tid = threadIdx.x;
-    const double INF = __longlong_as_double(0x7ff0000000000000LL);
     for (int64_t row = blockIdx.x; row < d; row += gridDim.x) {
         __syncthreads();
         for (int n = tid; n < NP2; n += blockDim.x) {
-            double u = INF;
+            uint64_t key = ~0ull;                                               // padding: after NaN keys (index >= N)
             if (n < N) {
                 const double nr = sqrt(__ldg(n2 + n));
-                u = __ldg(X + (int64_t)n * ld + row) / nr;                       // U[j,n] = X[j,n] / Xnorms[n]   :266
+                double u = __ldg(X + (int64_t)n * ld + row) / nr;                // U[j,n] = X[j,n] / Xnorms[n]   :266
                 if (kind == 2) u = (__ldg(sgn + n) * nr) * u;
+                key = sel_order(u);
             }
-            kk[n] = u;
+            kk[n] = key;
             ii[n] = n;
         }
         __syncthreads();
@@ -469,7 +472,7 @@ ga_robust_big_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, in
                     const int a = 2 * t - (t & (j - 1));
                     const int b = a + j;
                     const bool up = (a & k) == 0;
-                    const double ka = kk[a], kb = kk[b];
+                    const uint64_t ka = kk[a], kb = kk[b];
                     const int ia = ii[a], ib = ii[b];
                     const bool gt = (ka > kb) || (ka == kb && ia > ib);
                     if (gt == up) { kk[a] = kb; kk[b] = ka; ii[a] = ib; ii[b] = ia; }
@@ -481,7 +484,7 @@ ga_robust_big_kernel(const double* __restrict__ X, int64_t d, int N, int NP2, in
             for (int p = lo + tid; p < hi; p += blockDim.x) {
                 const int n = ii[p];
                 const double w = __ldg(sgn + n) * sqrt(__ldg(n2 + n));
-                num = fma(w, kk[p], num);
+                num = fma(w, sel_value(kk[p]), num);                             // w_n U[j,n]
                 den += w;
             }
             num = warp_sum(num);
@@ -667,12 +670,9 @@ cudaError_t launch_ga_robust(const double* X, int64_t d, int64_t N, int64_t ld, 
         if (launches) *launches += 1;
         return cudaGetLastError();
     }
-    static size_t attr = 0;
-    if (smem > attr) {
-        cudaError_t e = cudaFuncSetAttribute(ga_robust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        attr = smem;
-    }
+    // function attributes are per device: set on every launch (a process may run on several GPUs)
+    cudaError_t e = cudaFuncSetAttribute(ga_robust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
     const int lo = (int)floor(P * (double)N), hi = (int)floor((1.0 - P) * (double)N);      // :325
     int64_t blocks = (d + rt - 1) / rt;
     if (blocks > (int64_t)sm_count * 2) blocks = (int64_t)sm_count * 2;

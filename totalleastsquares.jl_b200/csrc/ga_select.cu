@@ -30,7 +30,8 @@ constexpr int SEL_UNROLL = 8;
 
 // Where the keys come from.  n2 == nullptr: X already holds U and wt the weights w_n.  Otherwise (rpca_ga) X is the
 // deflated data, u = X[j,n] / sqrt(n2[n]) and w_n = wt[n] sqrt(n2[n]) with wt the signs -- the same expressions as
-// ga_robust_kernel, so the orders agree on both sides of kGaRobustMaxN.
+// ga_robust_kernel, and the same key map sel_order, so the orders agree on both sides of kGaRobustMaxN
+// (tests/test_gpu_ga_paths.py checks N = 16 384 and 16 385 on the same data kinds).
 struct SelSrc {
     const double* X;
     int64_t ld;
@@ -95,14 +96,7 @@ size_t sel_layout(int64_t d, const SelPlan& p, void* base, SelWs* w) {
     return total;
 }
 
-// order-preserving map double -> uint64: -0.0 == +0.0, every NaN above +inf
-__device__ __forceinline__ uint64_t sel_order(double u) {
-    uint64_t b = (uint64_t)__double_as_longlong(u);
-    if ((b << 1) == 0) b = 0;                                              // -0.0 -> +0.0
-    if ((b & 0x7fffffffffffffffull) > 0x7ff0000000000000ull) return ~0ull;   // NaN: last (Julia's isless)
-    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-}
-
+// keys: sel_order (common.cuh), shared with the per-row sorts in ga.cu
 __device__ __forceinline__ void sel_uw(const SelSrc& s, int64_t n, double x, double& u, double& w) {
     const double nr = s.n2 ? sqrt(__ldg(s.n2 + n)) : 1.0;
     u = x / nr;                                                            // U[j,n] = X[j,n] / Xnorms[n]   :266

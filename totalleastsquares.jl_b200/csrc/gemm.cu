@@ -157,12 +157,9 @@ bool gemm_xb_eligible(const double* X, int64_t M, int K, int64_t ldx, int N) {
 cudaError_t launch_gemm_xb(const double* X, int64_t M, int K, int64_t ldx, const double* B, int N, double* C,
                            cudaStream_t st, int64_t* launches) {
     const size_t smem = (size_t)(2 * GK * XRS + 2 * GT * BKS) * sizeof(double);     // 33792 + 40960 = 74752 B
-    static bool set = false;
-    if (!set) {
-        cudaError_t e = cudaFuncSetAttribute(gemm_xb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        set = true;
-    }
+    // function attributes are per device: set on every launch (a process may run on several GPUs)
+    cudaError_t e = cudaFuncSetAttribute(gemm_xb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
     dim3 grid((unsigned)((M + GT - 1) / GT), (unsigned)((N + GT - 1) / GT));
     gemm_xb_kernel<<<grid, 256, smem, st>>>(X, M, K, ldx, B, N, C);
     if (launches) *launches += 1;

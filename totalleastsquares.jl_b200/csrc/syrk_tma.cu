@@ -341,14 +341,11 @@ cudaError_t launch_syrk_tma(const double* X, int64_t M, int64_t N, int64_t ld, c
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
     const size_t smem = (size_t)SST * STAGE_BYTES;
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        attr_set = true;
-    }
+    // function attributes are per device: set on every launch (a process may run on several GPUs)
+    cudaError_t e = cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
     syrk_tma_kernel<<<plan.ncta, 256, smem, st>>>(map, partial, plan);
-    cudaError_t e = cudaGetLastError();
+    e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int64_t nn = N * N;
     syrk_reduce_kernel<<<(unsigned)((nn + 255) / 256), 256, 0, st>>>(partial, plan, (int)N, G);
