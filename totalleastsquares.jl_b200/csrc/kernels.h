@@ -39,7 +39,7 @@ cudaError_t launch_gram(const GramSrc& s, GramMode mode, bool hankel, const Gram
 cudaError_t launch_gram_reduce(const double* partial, int nsplit, int nblk, int nb, int B, int N, double* G,
                                cudaStream_t st);
 
-// TMA-fed SYRK for a materialised dense X (syrk_tma.cu): 128 x 128 blocks, 16-row boxes, 4-stage mbarrier ring
+// TMA-fed SYRK for a materialised dense X (syrk_tma.cu): 128 x 128 blocks, 16-row boxes, 6-stage mbarrier ring
 constexpr int kSyrkBlk = 128;
 constexpr int kEigMaxN = 2048;              // largest min(M, N): 16 x 16 blocks of 128 columns
 constexpr int kEigSmallN = 512;             // up to here: shared-memory / register-resident eigen kernels (eig.cu, eig_fast.cu)

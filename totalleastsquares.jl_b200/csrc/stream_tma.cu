@@ -4,13 +4,13 @@
 //   alm_ew_tma_kernel  E_k, A_k = clamp(T_k V_k'), Z, Y_k, ||Z||_F^2, W_{k+1}       src/robustPCA.jl:188-192, 205-222
 //                      one read of D and Y_{k-1}, one write of Y_k and W_{k+1}
 //
-// Same arithmetic, operation order and thread <-> row mapping as alm_stream_kernel (stream.cu); what changes is the data
-// path.  The register-prefetch version is bound by load latency (ncu: 38 % of the stall samples sit on the first DFMA
-// that consumes a global load, 24 % warps active at 122 registers) and reaches 4.2 - 4.8 TB/s.  Here every CTA streams
-// 512-row x 8 (W) or 4 (D, Y) column boxes through a 4-stage ring of shared-memory buffers filled by TMA
-// (cp.async.bulk.tensor.2d, completion on mbarriers): 64 KB in flight per CTA without a single register or warp spent
-// on it, the threads only ever wait on shared memory.  512 threads per CTA (thread <-> row, 16 warps per SM) keep the
-// FP64 pipe fed; the inner loops are branch-free (out-of-range rows arrive zero-filled, only the stores are predicated).
+// Same per-element arithmetic and operation order as alm_stream_kernel (stream.cu); what changes is the data path.  The
+// register-prefetch version is bound by load latency (ncu: 38 % of the stall samples sit on the first DFMA that
+// consumes a global load, 24 % warps active at 122 registers) and reaches 4.2 - 4.8 TB/s.  Here every CTA streams
+// 32 KB stages of 256-row x 4-column boxes through a ring of up to 6 shared-memory buffers filled by TMA
+// (cp.async.bulk.tensor.2d, completion on mbarriers) without a single register or warp spent on it, the threads only
+// ever wait on shared memory.  Each thread owns two rows, so every shared-memory load of a V row feeds two elements;
+// the inner loops are branch-free (out-of-range rows arrive zero-filled, only the stores are predicated).
 #include <cuda.h>
 
 #include "kernels.h"
@@ -20,8 +20,8 @@ namespace tlsq {
 namespace {
 
 constexpr int TRB = 256;     // rows per TMA box
-constexpr int TT = 512;      // rows per tile == threads per CTA (thread <-> row): 16 warps per SM keep the FP64 pipe fed
-constexpr int TS = 4;        // ring stages (the launcher may use fewer)
+constexpr int TT = 512;      // rows per tile of the element-wise pass; threads per CTA of the projection
+constexpr int TS = 6;        // ring stages (the launcher uses as many as fit beside the V blocks)
 constexpr int TC2 = 4;       // columns per stage, element-wise pass (stage = D + Y = 32 KB)
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -174,9 +174,33 @@ tproj_tma_kernel(const __grid_constant__ CUtensorMap mW, const EpiArgs a, int sv
 // ---------------------------------------------------------------------------------------------------------------------
 // element-wise pass with both iterates factored (A_{k-1} = clamp(T_{k-1} V_{k-1}'), A_k = clamp(T_k V_k')).
 // Work unit = (tile, 4-column stage); the units are split evenly over the CTAs (a CTA may start in the middle of a tile).
+// Every thread owns TWO rows (tid and tid + EWT of a 2 EWT-row tile), so each broadcast LDS.128 of a V row feeds two
+// elements: the one-row form spent 14 of its ~75 instructions per element on those loads.
 // ---------------------------------------------------------------------------------------------------------------------
+constexpr int EWT = 256;                  // threads per CTA of the element-wise pass
+static_assert(PR * EWT == TT, "the element-wise tile is TT rows");
+
+// dot_rp for the two rows of a thread: the same two FMA chains and final add per row, one load of each V pair
+template <int RP>
+__device__ __forceinline__ void dot_rp2(const double (&t)[PR][RP], const double* __restrict__ v, double (&r)[PR]) {
+    double a0[PR], a1[PR];
+#pragma unroll
+    for (int p = 0; p < PR; ++p) a0[p] = a1[p] = 0.0;
+#pragma unroll
+    for (int c = 0; c < RP; c += 2) {
+        const double2 vv = *reinterpret_cast<const double2*>(v + c);
+#pragma unroll
+        for (int p = 0; p < PR; ++p) {
+            a0[p] = fma(t[p][c], vv.x, a0[p]);
+            a1[p] = fma(t[p][c + 1], vv.y, a1[p]);
+        }
+    }
+#pragma unroll
+    for (int p = 0; p < PR; ++p) r[p] = a0[p] + a1[p];
+}
+
 template <int RP, bool HANKEL>
-__global__ void __launch_bounds__(TT, 1)
+__global__ void __launch_bounds__(EWT, 1)
 alm_ew_tma_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__ CUtensorMap mY, const EpiArgs a,
                   int svp_host, const int* __restrict__ svp_dev, int ntiles, int nstage) {
     const int svp = svp_dev ? __ldg(svp_dev) : svp_host;
@@ -196,7 +220,7 @@ alm_ew_tma_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant_
         for (int s = 0; s < TS; ++s) mbar_init(&full[s], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    for (int idx = tid; idx < N * RP; idx += TT) {
+    for (int idx = tid; idx < N * RP; idx += EWT) {
         const int j = idx % N, c = idx / N;
         Vsm[j * RP + c] = c < svp ? __ldg(a.Vs + (int64_t)c * N + j) : 0.0;
         Vpm[j * RP + c] = c < a.svp_prev ? __ldg(a.Vp + (int64_t)c * N + j) : 0.0;
@@ -218,63 +242,79 @@ alm_ew_tma_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant_
     };
     if (tid == 0)
         for (int q = 0; q < nstage && q < total; ++q) issue(q, q);
-    double tr[RP], tp[RP];
-    double zz = 0.0;
-    int64_t row = 0;
-    bool rowok = false;
+    double tr[PR][RP], tp[PR][RP];
+    double zz[PR] = {};                                        // per row: the grouping of the one-row-per-thread form
+    int64_t row[PR];
+    bool rowok[PR];
     int s = 0;
     uint32_t phase = 0;
     int tile = (int)(g0 / nch), ch = (int)(g0 % nch);
     for (int q = 0; q < total; ++q) {
         if (q == 0 || ch == 0) {
-            row = (int64_t)tile * TT + tid;
-            rowok = row < a.M;
 #pragma unroll
-            for (int c = 0; c < RP; ++c) {
-                tr[c] = (rowok && c < svp) ? __ldg(a.Tn + (int64_t)c * a.M + row) : 0.0;
-                tp[c] = (rowok && c < a.svp_prev) ? __ldg(a.Tp + (int64_t)c * a.M + row) : 0.0;
+            for (int p = 0; p < PR; ++p) {
+                row[p] = (int64_t)tile * TT + tid + p * EWT;
+                rowok[p] = row[p] < a.M;
+#pragma unroll
+                for (int c = 0; c < RP; ++c) {
+                    tr[p][c] = (rowok[p] && c < svp) ? __ldg(a.Tn + (int64_t)c * a.M + row[p]) : 0.0;
+                    tp[p][c] = (rowok[p] && c < a.svp_prev) ? __ldg(a.Tp + (int64_t)c * a.M + row[p]) : 0.0;
+                }
             }
         }
         const int j0 = ch * TC2;
-        double dv[TC2], yv[TC2];
+        double dv[PR][TC2], yv[PR][TC2];
         if (HANKEL) {
 #pragma unroll
-            for (int u = 0; u < TC2; ++u) dv[u] = rowok ? src_at<true>(a.D, row, j0 + u) : 0.0;
+            for (int p = 0; p < PR; ++p)
+#pragma unroll
+                for (int u = 0; u < TC2; ++u) dv[p][u] = rowok[p] ? src_at<true>(a.D, row[p], j0 + u) : 0.0;
         }
         mbar_wait(&full[s], phase);
         const double* st = stage + s * STG;
 #pragma unroll
-        for (int u = 0; u < TC2; ++u) {
-            if (!HANKEL) dv[u] = stage_at<TC2>(st, tid, u);
-            yv[u] = stage_at<TC2>(st + HALF, tid, u);
-        }
-        double yn[TC2], w2[TC2], zv[TC2], ev[TC2];
+        for (int p = 0; p < PR; ++p)
+#pragma unroll
+            for (int u = 0; u < TC2; ++u) {
+                if (!HANKEL) dv[p][u] = stage_at<TC2>(st, tid + p * EWT, u);
+                yv[p][u] = stage_at<TC2>(st + HALF, tid + p * EWT, u);
+            }
+        double yn[PR][TC2], w2[PR][TC2], zv[PR][TC2], ev[PR][TC2];
 #pragma unroll
         for (int u = 0; u < TC2; ++u) {
             const int j = j0 + u;
-            const double d = dv[u], yp = yv[u];
-            double an = dot_rp<RP>(tr, Vsm + j * RP);
-            if (a.nonnegA) an = (__double_as_longlong(an) > 0) ? an : 0.0;           // A .= max.(A, 0)   :218
-            double ap = dot_rp<RP>(tp, Vpm + j * RP);                                // A_{k-1} from its factors
-            if (a.nonnegA) ap = (__double_as_longlong(ap) > 0) ? ap : 0.0;
-            double e, w;
-            alm_ew(d, ap, yp, a.im, a.eps, a.nonnegE, e, w);
-            const double z = __dsub_rn(__dsub_rn(d, an), e);                          // @. Z = D - A - E  :221
-            yn[u] = __dadd_rn(yp, __dmul_rn(a.mu, z));                                // @. Y = Y + mu*Z   :222
-            zz = fma(z, z, zz);                                                       // (rows beyond M are all-zero)
-            zv[u] = z;
-            ev[u] = e;
-            double e2;
-            alm_ew(d, an, yn[u], a.im_next, a.eps_next, a.nonnegE, e2, w2[u]);        // SVT input of iteration k+1
-        }
-        if (rowok) {
+            double an[PR], ap[PR];
+            dot_rp2<RP>(tr, Vsm + j * RP, an);
+            dot_rp2<RP>(tp, Vpm + j * RP, ap);                                       // A_{k-1} from its factors
 #pragma unroll
-            for (int u = 0; u < TC2; ++u) {
-                const int64_t off = (int64_t)(j0 + u) * a.ldw + row;
-                a.Yn[off] = yn[u];
-                a.Wn[off] = w2[u];
-                if (a.Eout) a.Eout[off] = ev[u];
-                if (a.Zout) a.Zout[off] = zv[u];
+            for (int p = 0; p < PR; ++p) {
+                if (a.nonnegA) {                                                      // A .= max.(A, 0)   :218
+                    an[p] = (__double_as_longlong(an[p]) > 0) ? an[p] : 0.0;
+                    ap[p] = (__double_as_longlong(ap[p]) > 0) ? ap[p] : 0.0;
+                }
+                const double d = dv[p][u], yp = yv[p][u];
+                double e, w;
+                alm_ew(d, ap[p], yp, a.im, a.eps, a.nonnegE, e, w);
+                const double z = __dsub_rn(__dsub_rn(d, an[p]), e);                   // @. Z = D - A - E  :221
+                yn[p][u] = __dadd_rn(yp, __dmul_rn(a.mu, z));                         // @. Y = Y + mu*Z   :222
+                zz[p] = fma(z, z, zz[p]);                                             // (rows beyond M are all-zero)
+                zv[p][u] = z;
+                ev[p][u] = e;
+                double e2;
+                alm_ew(d, an[p], yn[p][u], a.im_next, a.eps_next, a.nonnegE, e2, w2[p][u]);   // SVT input of k+1
+            }
+        }
+#pragma unroll
+        for (int p = 0; p < PR; ++p) {
+            if (rowok[p]) {
+#pragma unroll
+                for (int u = 0; u < TC2; ++u) {
+                    const int64_t off = (int64_t)(j0 + u) * a.ldw + row[p];
+                    a.Yn[off] = yn[p][u];
+                    a.Wn[off] = w2[p][u];
+                    if (a.Eout) a.Eout[off] = ev[p][u];
+                    if (a.Zout) a.Zout[off] = zv[p][u];
+                }
             }
         }
         // refill only after the values read from the stage have been consumed (see tproj_tma_kernel)
@@ -283,8 +323,12 @@ alm_ew_tma_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant_
         if (++s == nstage) { s = 0; phase ^= 1u; }
         if (++ch == nch) { ch = 0; ++tile; }
     }
-    zz = warp_sum(zz);
-    if ((tid & 31) == 0) red[tid >> 5] = zz;
+    // rows tid + p * EWT: warp w's sums of p = 0 and 1 are those of rows [32 w, +32) and [EWT + 32 w, +32)
+#pragma unroll
+    for (int p = 0; p < PR; ++p) {
+        const double v = warp_sum(zz[p]);
+        if ((tid & 31) == 0) red[p * (EWT / 32) + (tid >> 5)] = v;
+    }
     __syncthreads();
     if (tid == 0) {
         double t = 0.0;
@@ -337,6 +381,7 @@ cudaError_t launch_rp(const EpiArgs& a, const double* W, int svp, const int* svp
     const size_t stage_bytes = (size_t)TC1 * TT1 * 8;                      // == 2 * TC2 * TT * 8 == 32 KB
     const size_t v1 = (size_t)a.N * RP * 8, v2 = 2 * v1;
     int ns1 = TS, ns2 = TS;
+    while (ns1 > 2 && ns1 * stage_bytes + v1 > (size_t)220 * 1024) --ns1;
     while (ns2 > 2 && ns2 * stage_bytes + v2 > (size_t)220 * 1024) --ns2;
     const size_t sm1 = ns1 * stage_bytes + v1, sm2 = ns2 * stage_bytes + v2;
     int grid = sm_count < ntiles1 ? sm_count : ntiles1;
@@ -350,11 +395,11 @@ cudaError_t launch_rp(const EpiArgs& a, const double* W, int svp, const int* svp
     if (hankel) {
         auto kern = alm_ew_tma_kernel<RP, true>;
         if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm2)) != cudaSuccess) return e;
-        kern<<<sm_count, TT, sm2, st>>>(mD, mY, a, svp, svp_dev, ntiles, ns2);
+        kern<<<sm_count, EWT, sm2, st>>>(mD, mY, a, svp, svp_dev, ntiles, ns2);
     } else {
         auto kern = alm_ew_tma_kernel<RP, false>;
         if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm2)) != cudaSuccess) return e;
-        kern<<<sm_count, TT, sm2, st>>>(mD, mY, a, svp, svp_dev, ntiles, ns2);
+        kern<<<sm_count, EWT, sm2, st>>>(mD, mY, a, svp, svp_dev, ntiles, ns2);
     }
     return cudaGetLastError();
 }

@@ -2,12 +2,13 @@
 //
 // This is the hot Gram pass of the ALM loop once the SVT input W_k is materialised by the previous epilogue
 // (replaces LAPACK dgesdd of src/robustPCA.jl:194; also used for opnorm(D), :177).  Blackwell-native data path:
-//   * TMA (cp.async.bulk.tensor.2d, SASS UTMALDG) streams 16-row x 128-column boxes of X into a 4-stage shared
-//     memory ring, completion signalled on mbarriers (no register staging, 128 KB in flight per SM);
+//   * TMA (cp.async.bulk.tensor.2d, SASS UTMALDG) streams 16-row x 128-column boxes of X into a 6-stage shared
+//     memory ring, completion signalled on mbarriers (no register staging, 192 KB of ring per SM); each warp releases
+//     a stage on a second mbarrier when it is done with it, and no CTA-wide barrier paces the warps;
 //   * the boxes land with the hardware 128-byte swizzle; together with a permuted k order inside each 16-row
 //     tile (lane t takes k = 2s + (t&1) + 8(t>>1)) every 8-byte DMMA fragment load of a half-warp hits 16
 //     distinct banks -- no padding, no conflicts;
-//   * 8 warps in a 4 x 2 layout own a 128 x 128 output block, warp tile 32 x 64 = 32 DMMA.8x8x4 accumulators
+//   * 8 compute warps in a 4 x 2 layout own a 128 x 128 output block, warp tile 32 x 64 = 32 DMMA.8x8x4 accumulators
 //     (64 FP64 registers pairs) per k-step, FP64 tensor pipe (mma.sync.m8n8k4.f64; tcgen05 has no FP64 kind).
 // grid.x enumerates the upper-triangular 128-blocks (bi <= bj), grid.y splits the rows; CTAs of one split stream
 // the same rows at the same time so the panels shared between blocks are served by L2.  Partial blocks are
@@ -21,12 +22,11 @@ namespace tlsq {
 namespace {
 
 constexpr int SB = kSyrkBlk;      // 128 output block edge
-constexpr int SR = 16;            // rows per TMA box (128-byte inner extent = the swizzle span)
-constexpr int SRS = 32;           // rows per pipeline stage (two boxes per panel)
-constexpr int SST = 3;            // pipeline stages
+constexpr int SR = 16;            // rows per TMA box (128-byte inner extent = the swizzle span) and per ring stage
+constexpr int SRS = 32;           // rows per tile: the unit the row splits are dealt in
+constexpr int SST = 6;            // ring stages (three tiles)
 constexpr int BOX_BYTES = SB * SR * 8;         // 16 KB
-constexpr int PANEL_BYTES = 2 * BOX_BYTES;     // 32 KB: 32 rows x 128 columns
-constexpr int STAGE_BYTES = 2 * PANEL_BYTES;   // 64 KB: panel i + panel j
+constexpr int STAGE_BYTES = 2 * BOX_BYTES;     // 32 KB: box of panel i + box of panel j (diagonal blocks: panel i only)
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -35,6 +35,9 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     uint32_t done;
@@ -55,61 +58,70 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
 }
 
 // Warp -> output tiles.  Off-diagonal block: 4 x 2 warps, warp tile 32 x 64 (32 DMMA accumulators).  Diagonal block:
-// only the 10 upper 32 x 32 tiles are computed; they are cut into 40 strips of 32 x 8 columns, enumerated tile row by
-// tile row, and warp w takes strips [5w, 5w + 5) -- 20 DMMAs per k-step on every warp (perfectly balanced, a diagonal
-// block costs 5/8 of an off-diagonal one and gets proportionally fewer CTAs, see syrk_plan).  A warp's strips span at
-// most two tile rows: the first n1 take their A fragments from tile row rowA, the others from rowB.
-struct DiagStrips { int rowA, rowB, n1; int cs[5]; };
-__device__ __forceinline__ DiagStrips diag_strips(int warp) {
-    DiagStrips d;
-    int n = 0, k = 0;
-    d.rowA = d.rowB = 0; d.n1 = 0;
-#pragma unroll
+// only the 8 x 8 tiles on or above the diagonal are computed -- the 6 upper off-diagonal 32 x 32 tiles in full and the
+// upper triangles (1 + 2 + 3 + 4 tiles) of the 4 diagonal ones, 136 tiles.  They are enumerated by 32-row tile row,
+// then 8-column strip, then row inside the strip, and warp w takes tiles [17w, 17w + 17): 17 DMMAs per k-step on every
+// warp.  Both operands of a diagonal block come from the same panel, so a tile (r8, c8) reads fragments r8 and c8 of it.
+constexpr int DT = 17;                                    // 8 x 8 tiles per warp in a diagonal block
+struct DiagMap { int r8[DT], c8[DT]; uint32_t frags; };   // frags: bit f = fragment f is read by this warp
+__host__ __device__ constexpr DiagMap diag_map(int warp) {
+    DiagMap m{};
+    int n = 0;
     for (int arow = 0; arow < 4; ++arow)
-#pragma unroll
-        for (int c = 4 * arow; c < 16; ++c, ++n) {
-            if (n >= 5 * warp && n < 5 * warp + 5) {
-                if (k == 0) d.rowA = arow;
-                d.rowB = arow;
-                if (arow == d.rowA) d.n1 = k + 1;
-                d.cs[k++] = c;
-            }
+        for (int c = 4 * arow; c < 16; ++c) {
+            const int h = (c >> 2) == arow ? (c & 3) + 1 : 4;     // rows of the strip on or above the diagonal
+            for (int mi = 0; mi < h; ++mi, ++n)
+                if (n >= DT * warp && n < DT * warp + DT) {
+                    m.r8[n - DT * warp] = 4 * arow + mi;
+                    m.c8[n - DT * warp] = c;
+                    m.frags |= (1u << (4 * arow + mi)) | (1u << c);
+                }
         }
-    return d;
+    return m;
 }
+static_assert(diag_map(7).c8[DT - 1] == 15 && diag_map(7).r8[DT - 1] == 15, "136 tiles over 8 warps");
 
-// the first N1 strips use a1, the others a2 (N1 is per-warp constant: the switch keeps accumulator indexing static)
-template <int N1>
-__device__ __forceinline__ void diag_stage(double (&acc)[4][8][2], const uint8_t* pa, uint32_t aA, uint32_t aB,
-                                           const uint32_t (&bo)[5], const uint32_t (&koff)[4]) {
+template <int W>
+__device__ __forceinline__ void diag_stage(double (&acc)[4][8][2], const uint8_t* pa, uint32_t fcol,
+                                           const uint32_t (&koff)[4]) {
+    constexpr DiagMap m = diag_map(W);
 #pragma unroll
-    for (int half = 0; half < 2; ++half) {
-        const uint8_t* ph = pa + half * BOX_BYTES;
+    for (int s4 = 0; s4 < 4; ++s4) {
+        double f[16];
 #pragma unroll
-        for (int s4 = 0; s4 < 4; ++s4) {
-            double a1[4], a2[4];
+        for (int q = 0; q < 16; ++q)
+            if ((m.frags >> q) & 1u) f[q] = *reinterpret_cast<const double*>(pa + fcol + (uint32_t)q * 1024u + koff[s4]);
 #pragma unroll
-            for (int mi = 0; mi < 4; ++mi) {
-                a1[mi] = *reinterpret_cast<const double*>(ph + aA + (uint32_t)mi * 1024u + koff[s4]);
-                if (N1 < 5) a2[mi] = *reinterpret_cast<const double*>(ph + aB + (uint32_t)mi * 1024u + koff[s4]);
-            }
-#pragma unroll
-            for (int s = 0; s < 5; ++s) {
-                const double b = *reinterpret_cast<const double*>(ph + bo[s] + koff[s4]);
-#pragma unroll
-                for (int mi = 0; mi < 4; ++mi) dmma884(acc[mi][s][0], acc[mi][s][1], s < N1 ? a1[mi] : a2[mi], b);
-            }
-        }
+        for (int k = 0; k < DT; ++k) dmma884(acc[k >> 3][k & 7][0], acc[k >> 3][k & 7][1], f[m.r8[k]], f[m.c8[k]]);
     }
 }
 
-__global__ void __launch_bounds__(256, 1)
+template <int W>
+__device__ __forceinline__ void diag_store(const double (&acc)[4][8][2], double* P, int g, int t) {
+    constexpr DiagMap m = diag_map(W);
+#pragma unroll
+    for (int k = 0; k < DT; ++k) {
+        const int il = 8 * m.r8[k] + g, jl = 8 * m.c8[k] + 2 * t;
+        P[jl * SB + il] = acc[k >> 3][k & 7][0];
+        P[(jl + 1) * SB + il] = acc[k >> 3][k & 7][1];
+    }
+}
+
+// A stage is refilled once all 8 warps have arrived on its "empty" mbarrier, and a warp arrives only after its last
+// fragment read from the stage has gone into a DMMA (the fragments are register operands of the asm DMMAs, which stay
+// ahead of the asm arrive): an LDS still in flight is not ordered against the TMA engine's write of the refill (see
+// DESIGN §4).  Thread 0 refills one stage late -- after consuming stage i it waits for stage i - 1 to be released,
+// which the other warps have normally done by then -- and the other warps never wait for each other.  A dedicated
+// producer warp would cap the registers at 168 (three warps on one SM sub-partition) and spill the accumulators.
+constexpr int SWARPS = 8;
+
+__global__ void __launch_bounds__(32 * SWARPS, 1)
 syrk_tma_kernel(const __grid_constant__ CUtensorMap tmap, double* __restrict__ partial,
                 const __grid_constant__ SyrkPlan plan) {
     // 1024-byte alignment is required by the 128B swizzle pattern.  The pointer is NOT re-aligned with integer
     // arithmetic: that would turn every fragment load into a generic LD instead of LDS.
     extern __shared__ __align__(1024) uint8_t smem_dyn[];
-    __shared__ uint64_t full_bar[SST];
+    __shared__ uint64_t full_bar[SST], empty_bar[SST];
     uint8_t* base = smem_dyn;
     if ((smem_u32(base) & 1023u) != 0u) __trap();
 
@@ -129,35 +141,32 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmap, double* __restrict__ p
     const bool diag = (bi == bj);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int g = lane >> 2, t = lane & 3;
-    const int a0 = 32 * (warp & 3), b0 = 64 * (warp >> 2);       // off-diagonal warp tile
-    const DiagStrips ds = diag_strips(warp);
 
     if (tid == 0) {
 #pragma unroll
-        for (int s = 0; s < SST; ++s) mbar_init(&full_bar[s], 1);
+        for (int s = 0; s < SST; ++s) {
+            mbar_init(&full_bar[s], 1);
+            mbar_init(&empty_bar[s], SWARPS);
+        }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
 
-    const int nmy = (plan.ntiles - split + nsplit - 1) / nsplit;       // 32-row tiles of this CTA
-    const uint32_t stage_tx = diag ? PANEL_BYTES : STAGE_BYTES;
-
+    // stage i = rows [16 (i & 1), +16) of this CTA's (i >> 1)-th 32-row tile
+    const int nst = 2 * ((plan.ntiles - split + nsplit - 1) / nsplit);
+    const uint32_t stage_tx = diag ? BOX_BYTES : STAGE_BYTES;
     auto issue = [&](int i) {
         const int s = i % SST;
-        const int kt = split + i * nsplit;
+        const int row = (split + (i >> 1) * nsplit) * SRS + (i & 1) * SR;
         uint8_t* st = base + (size_t)s * STAGE_BYTES;
         mbar_expect_tx(&full_bar[s], stage_tx);
-        tma_load_2d(st, &tmap, kt * SRS, bi * SB, &full_bar[s]);
-        tma_load_2d(st + BOX_BYTES, &tmap, kt * SRS + SR, bi * SB, &full_bar[s]);
-        if (!diag) {
-            tma_load_2d(st + PANEL_BYTES, &tmap, kt * SRS, bj * SB, &full_bar[s]);
-            tma_load_2d(st + PANEL_BYTES + BOX_BYTES, &tmap, kt * SRS + SR, bj * SB, &full_bar[s]);
-        }
+        tma_load_2d(st, &tmap, row, bi * SB, &full_bar[s]);
+        if (!diag) tma_load_2d(st + BOX_BYTES, &tmap, row, bj * SB, &full_bar[s]);
     };
-    if (tid == 0) {
-        for (int i = 0; i < SST && i < nmy; ++i) issue(i);
-    }
+    if (tid == 0)
+        for (int i = 0; i < SST && i < nst; ++i) issue(i);
 
+    const int a0 = 32 * (warp & 3), b0 = 64 * (warp >> 2);       // off-diagonal warp tile
     // per-lane swizzled byte offsets of the 4 k-steps:  k = 2s + (t&1) + 8(t>>1);  chunk16 = (k>>1) ^ (col&7), col&7 == g
     uint32_t koff[4];
 #pragma unroll
@@ -167,10 +176,7 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmap, double* __restrict__ p
     }
     const uint32_t a_col = (uint32_t)(a0 + g) * 128u;
     const uint32_t b_col = (uint32_t)(b0 + g) * 128u;
-    const uint32_t dA = (uint32_t)(32 * ds.rowA + g) * 128u, dB = (uint32_t)(32 * ds.rowB + g) * 128u;
-    uint32_t dbo[5];
-#pragma unroll
-    for (int s5 = 0; s5 < 5; ++s5) dbo[s5] = (uint32_t)(8 * ds.cs[s5] + g) * 128u;
+    const uint32_t f_col = (uint32_t)g * 128u;
 
     double acc[4][8][2];
 #pragma unroll
@@ -178,41 +184,45 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmap, double* __restrict__ p
 #pragma unroll
         for (int ni = 0; ni < 8; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
 
-    for (int i = 0; i < nmy; ++i) {
+    for (int i = 0; i < nst; ++i) {
         const int s = i % SST;
-        const uint32_t parity = (uint32_t)((i / SST) & 1);
-        mbar_wait(&full_bar[s], parity);
+        mbar_wait(&full_bar[s], (uint32_t)((i / SST) & 1));
         const uint8_t* pa = base + (size_t)s * STAGE_BYTES;
-        const uint8_t* pb = diag ? pa : pa + PANEL_BYTES;
         if (!diag) {
+            const uint8_t* pb = pa + BOX_BYTES;
 #pragma unroll
-            for (int half = 0; half < 2; ++half) {
+            for (int s4 = 0; s4 < 4; ++s4) {
+                double a[4], b[8];
 #pragma unroll
-                for (int s4 = 0; s4 < 4; ++s4) {
-                    double a[4], b[8];
+                for (int mi = 0; mi < 4; ++mi)
+                    a[mi] = *reinterpret_cast<const double*>(pa + a_col + (uint32_t)mi * 1024u + koff[s4]);
 #pragma unroll
-                    for (int mi = 0; mi < 4; ++mi)
-                        a[mi] = *reinterpret_cast<const double*>(pa + half * BOX_BYTES + a_col + (uint32_t)mi * 1024u + koff[s4]);
+                for (int ni = 0; ni < 8; ++ni)
+                    b[ni] = *reinterpret_cast<const double*>(pb + b_col + (uint32_t)ni * 1024u + koff[s4]);
 #pragma unroll
-                    for (int ni = 0; ni < 8; ++ni)
-                        b[ni] = *reinterpret_cast<const double*>(pb + half * BOX_BYTES + b_col + (uint32_t)ni * 1024u + koff[s4]);
+                for (int ni = 0; ni < 8; ++ni)
 #pragma unroll
-                    for (int ni = 0; ni < 8; ++ni)
-#pragma unroll
-                        for (int mi = 0; mi < 4; ++mi) dmma884(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
-                }
+                    for (int mi = 0; mi < 4; ++mi) dmma884(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
             }
         } else {
-            switch (ds.n1) {
-                case 1: diag_stage<1>(acc, pa, dA, dB, dbo, koff); break;
-                case 2: diag_stage<2>(acc, pa, dA, dB, dbo, koff); break;
-                case 3: diag_stage<3>(acc, pa, dA, dB, dbo, koff); break;
-                case 4: diag_stage<4>(acc, pa, dA, dB, dbo, koff); break;
-                default: diag_stage<5>(acc, pa, dA, dB, dbo, koff); break;
+            switch (warp) {
+                case 0: diag_stage<0>(acc, pa, f_col, koff); break;
+                case 1: diag_stage<1>(acc, pa, f_col, koff); break;
+                case 2: diag_stage<2>(acc, pa, f_col, koff); break;
+                case 3: diag_stage<3>(acc, pa, f_col, koff); break;
+                case 4: diag_stage<4>(acc, pa, f_col, koff); break;
+                case 5: diag_stage<5>(acc, pa, f_col, koff); break;
+                case 6: diag_stage<6>(acc, pa, f_col, koff); break;
+                default: diag_stage<7>(acc, pa, f_col, koff); break;
             }
         }
-        __syncthreads();                               // every warp is done with stage s -> refill it
-        if (tid == 0 && i + SST < nmy) issue(i + SST);
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty_bar[s]);
+        if (tid == 0 && i >= 1 && i - 1 + SST < nst) {
+            const int r = i - 1;
+            mbar_wait(&empty_bar[r % SST], (uint32_t)((r / SST) & 1));
+            issue(r + SST);
+        }
     }
 
     double* P = partial + ((size_t)plan.part_off[blk] + split) * (SB * SB);
@@ -227,21 +237,21 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmap, double* __restrict__ p
                 P[(jl + 1) * SB + il] = acc[mi][ni][1];
             }
     } else {
-#pragma unroll
-        for (int s5 = 0; s5 < 5; ++s5) {
-            const int ra = 32 * (s5 < ds.n1 ? ds.rowA : ds.rowB);
-#pragma unroll
-            for (int mi = 0; mi < 4; ++mi) {
-                const int il = ra + 8 * mi + g;
-                const int jl = 8 * ds.cs[s5] + 2 * t;
-                P[jl * SB + il] = acc[mi][s5][0];
-                P[(jl + 1) * SB + il] = acc[mi][s5][1];
-            }
+        switch (warp) {
+            case 0: diag_store<0>(acc, P, g, t); break;
+            case 1: diag_store<1>(acc, P, g, t); break;
+            case 2: diag_store<2>(acc, P, g, t); break;
+            case 3: diag_store<3>(acc, P, g, t); break;
+            case 4: diag_store<4>(acc, P, g, t); break;
+            case 5: diag_store<5>(acc, P, g, t); break;
+            case 6: diag_store<6>(acc, P, g, t); break;
+            default: diag_store<7>(acc, P, g, t); break;
         }
     }
 }
 
-// G[i,j] = G[j,i] = sum over the splits of block(i,j), fixed order; diagonal blocks only hold their upper 32-tiles
+// G[i,j] = G[j,i] = sum over the splits of block(i,j), fixed order; diagonal blocks only hold their 8 x 8 tiles on or
+// above the diagonal, which cover every (il, jl) with il <= jl
 __global__ void syrk_reduce_kernel(const double* __restrict__ partial, const __grid_constant__ SyrkPlan plan, int N,
                                    double* __restrict__ G) {
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -249,8 +259,7 @@ __global__ void syrk_reduce_kernel(const double* __restrict__ partial, const __g
     int i = (int)(idx % N), j = (int)(idx / N);
     if (i > j) return;
     const int bi = i / SB, bj = j / SB;
-    int il = i % SB, jl = j % SB;
-    if (bi == bj && (il >> 5) > (jl >> 5)) return;      // cannot happen for i <= j; kept for clarity
+    const int il = i % SB, jl = j % SB;
     const int blk = bi * plan.nb - (bi * (bi - 1)) / 2 + (bj - bi);
     const double* p = partial + (size_t)plan.part_off[blk] * (SB * SB) + jl * SB + il;
     double sum = 0.0;
@@ -295,13 +304,18 @@ SyrkPlan syrk_plan(int64_t M, int64_t N, int sm_count) {
     p.nb = (int)((N + SB - 1) / SB);
     p.nblk = p.nb * (p.nb + 1) / 2;
     p.ntiles = (int)((M + SRS - 1) / SRS);
-    // CTAs per block proportional to the block's cost (off-diagonal: 32 DMMAs per warp and k-step, diagonal: 20)
+    // CTAs per block roughly proportional to the block's cost (off-diagonal: 32 DMMAs per warp and k-step, diagonal: 17).
+    // The diagonal weight stays at the 20 / 32 of the kernel that computed whole 32 x 32 diagonal tiles: a split's rows
+    // fix the partial sum, and weighting by 17 / 32 would move rows between partial sums.  G would then change in its
+    // last bits, and so would the nearly degenerate trailing singular vectors of the returned SVD.  The diagonal CTAs
+    // finish early instead; the off-diagonal ones set the pace.
+    constexpr double kOff = 4.0, kDiag = 2.5;
     int ndiag = p.nb, noff = p.nblk - p.nb;
-    double unit = (double)sm_count / (4.0 * noff + 2.5 * ndiag);
+    double unit = (double)sm_count / (kOff * noff + kDiag * ndiag);
     int total = 0, blk = 0;
     for (int bi = 0; bi < p.nb; ++bi)
         for (int bj = bi; bj < p.nb; ++bj, ++blk) {
-            int ns = (int)((bi == bj ? 2.5 : 4.0) * unit);
+            int ns = (int)((bi == bj ? kDiag : kOff) * unit);
             if (ns < 1) ns = 1;
             if (ns > p.ntiles) ns = p.ntiles;
             p.nsplit_blk[blk] = ns;
@@ -344,7 +358,7 @@ cudaError_t launch_syrk_tma(const double* X, int64_t M, int64_t N, int64_t ld, c
     // function attributes are per device: set on every launch (a process may run on several GPUs)
     cudaError_t e = cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    syrk_tma_kernel<<<plan.ncta, 256, smem, st>>>(map, partial, plan);
+    syrk_tma_kernel<<<plan.ncta, 32 * SWARPS, smem, st>>>(map, partial, plan);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int64_t nn = N * N;
