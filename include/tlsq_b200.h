@@ -116,7 +116,7 @@ int tlsq_rpca_f64_dev(tlsq_handle* h, const double* D, int64_t M, int64_t N,
  * :225; reference test test/runtests.jl:384-398).  A Julia closure reaches the library as a C function pointer
  * (@cfunction) plus an opaque `user` pointer.  The matrices cross the boundary in HOST memory (column-major), so every
  * call costs a device->host and a host->device copy: this is the reference's plugin hook, not the fast path.  NULL
- * selects the built-in device implementation.  Single GPU, host pointers, any orientation, min(M,N) <= 2048.
+ * selects the built-in device implementation.  Single GPU, host pointers, any orientation, min(M,N) <= 4096.
  *  svd_fn   : thin or truncated SVD of Z (M x N): fill U (M x r, column-major), S (r, descending), Vt (r x N, leading
  *             dimension r) with 0 <= r <= min(M,N) and return r (< 0: error).  Called for k >= 2 with the current `sv`
  *             like the reference's svd(Z, sv) (:196); the first iteration always uses the built-in SVD (:193-194).
@@ -189,9 +189,15 @@ int tlsq_unhankel_mc_f64(tlsq_handle* h, const double* A, int64_t K, int64_t L, 
  * tlsq_plan_pipeline: the per-iteration pipeline every rank of a sharded solve derives from the rank-summed votes
  *   votes_sum = sum over ranks of {can run the two-kernel pipeline, can run the one-pass kernel, wants the one-pass
  *   kernel for memory, wants Y in place}; env_fused = -1 (unset) / 0 / 1 mirrors TLSQ_FUSED.
- * tlsq_plan_hankel_shard: rows [r0, r0 + Kl) of the K Hankel rows that `rank` owns in a sharded lowrankfilter.       */
+ * tlsq_plan_hankel_shard: rows [r0, r0 + Kl) of the K Hankel rows that `rank` owns in a sharded lowrankfilter.
+ * tlsq_plan_syrk: the CTA split of the TMA SYRK (G = X'X, X: M x N, 1 <= N <= 4096) on a device with sm_count SMs.
+ *   Upper-triangular 128 x 128 blocks b = 0 .. nblk-1 in row order (bi <= bj); block b runs on CTAs
+ *   [cta_begin[b], cta_begin[b+1]), nsplit_blk[b] of them, and sums into partial slots [part_off[b], +nsplit_blk[b]).
+ *   nsplit_blk and part_off need nb (nb + 1) / 2 entries with nb = ceil(N / 128), cta_begin one more.              */
 int tlsq_plan_pipeline(int nranks, const double* votes_sum, int env_fused, int* fused, int* use_w, int* inplace);
 int tlsq_plan_hankel_shard(int64_t K, int nranks, int rank, int64_t* r0, int64_t* Kl);
+int tlsq_plan_syrk(int64_t M, int64_t N, int sm_count, int* nblk, int* ncta, int* nsplit_blk, int* cta_begin,
+                   int* part_off, int64_t* partial_bytes);
 /* work split of the one-pass kernel's 256 x 256 Gram: tile_row / strip_col [2 CTAs][8 warps][9 strips] -- strip s of
  * warp w of CTA r is rows [32 tile_row, +32) x columns [8 strip_col, +8) of the upper triangle                      */
 int tlsq_plan_fused_strips(uint8_t* tile_row, uint8_t* strip_col);

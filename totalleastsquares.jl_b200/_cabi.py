@@ -63,6 +63,7 @@ SIGNATURES = {
                                      C.POINTER(C.c_int)]),
     "tlsq_plan_fused_strips": (C.c_int, [vp, vp]),
     "tlsq_plan_hankel_shard": (C.c_int, [C.c_int64, C.c_int, C.c_int, c_i64p, c_i64p]),
+    "tlsq_plan_syrk": (C.c_int, [C.c_int64, C.c_int64, C.c_int, vp, vp, vp, vp, vp, c_i64p]),
     "tlsq_gram_f64_dev": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp]),
     "tlsq_eigh_f64_dev": (C.c_int, [vp, vp, C.c_int64, vp, vp]),
     "tlsq_robust_average_f64_dev": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp, C.c_int, C.c_double, vp]),

@@ -294,8 +294,9 @@ jacobi_global_kernel(int n, int np, double tol, int max_sweeps, double* __restri
 
 
 // Same engine for large n (> 512): a column no longer fits a lane's registers, so every pair makes two passes over its
-// columns (dot products, then the rotation) out of L2.  Slow (O(100 ms) per sweep at n = 2048) but it is only the
-// fallback of the large-n fast path and the once-per-solve full spectrum of the returned SVD.
+// columns (dot products, then the rotation) out of L2.  Slow (O(100 ms) per sweep at n = 2048; above that Xo + Vo no
+// longer fit the L2, DESIGN §3.3) but it is only the fallback of the large-n fast path and the once-per-solve full
+// spectrum of the returned SVD.
 __global__ void __launch_bounds__(256)
 jacobi_global_loop_kernel(int n, int np, double tol, int max_sweeps, double* __restrict__ Xo, double* __restrict__ Vo,
                           int* __restrict__ info, const int* __restrict__ run_flag) {
@@ -698,6 +699,18 @@ cudaError_t launch_global(int n, int np, double tol, int max_sweeps, double* Xo,
     return cudaLaunchCooperativeKernel((void*)jacobi_global_kernel<E>, dim3(blocks), dim3(256), args, 0, st);
 }
 
+// eig_post_kernel keeps 2 ncols doubles in shared memory: above 48 KB (n > 3072) the launch needs the opt-in
+cudaError_t launch_eig_post(const double* Xo, const double* Vo, int n, int ncols, double* lam_raw, double* lam, int* perm,
+                            const int* run_flag, int svd_mode, cudaStream_t st) {
+    const size_t smem = 2 * (size_t)ncols * sizeof(double);
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(eig_post_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    eig_post_kernel<<<1, 256, smem, st>>>(Xo, Vo, n, ncols, lam_raw, lam, perm, run_flag, svd_mode);
+    return cudaGetLastError();
+}
+
 }  // namespace
 
 size_t eig_work_doubles(int n) {
@@ -758,9 +771,8 @@ cudaError_t launch_eigh(const double* G, int n, const double* V0, EigWork w, dou
         if ((e = cudaLaunchCooperativeKernel((void*)kern, dim3(C), dim3(256), args, smem, st)) != cudaSuccess) return e;
         if (launches) *launches += 2;
         // eig_post / permute read n-row columns from XoA / VoA
-        eig_post_kernel<<<1, 256, 2 * ncols * sizeof(double), st>>>(XoA, VoA, n, ncols, w.lam_raw, lam, w.perm, run_flag,
-                                                                     svd_mode);
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        if ((e = launch_eig_post(XoA, VoA, n, ncols, w.lam_raw, lam, w.perm, run_flag, svd_mode, st)) != cudaSuccess)
+            return e;
         permute_cols_kernel<<<n, 128, 0, st>>>(VoA, w.perm, n, Vs, run_flag);
         if (launches) *launches += 2;
         return cudaGetLastError();
@@ -774,16 +786,20 @@ cudaError_t launch_eigh(const double* G, int n, const double* V0, EigWork w, dou
         if (e != cudaSuccess) return e;
         if (launches) *launches += 2;
     }
-    eig_post_kernel<<<1, 256, 2 * ncols * sizeof(double), st>>>(w.Xo, w.Vo, n, ncols, w.lam_raw, lam, w.perm, run_flag,
-                                                                 svd_mode);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if ((e = launch_eig_post(w.Xo, w.Vo, n, ncols, w.lam_raw, lam, w.perm, run_flag, svd_mode, st)) != cudaSuccess)
+        return e;
     permute_cols_kernel<<<n, 128, 0, st>>>(w.Vo, w.perm, n, Vs, run_flag);
     if (launches) *launches += 2;
     return cudaGetLastError();
 }
 
 cudaError_t launch_chol_upper(double* R, int n, cudaStream_t st, int64_t* launches) {
-    chol_upper_kernel<<<1, 1024, 2 * (size_t)n * sizeof(double), st>>>(R, n);
+    const size_t smem = 2 * (size_t)n * sizeof(double);       // above 48 KB (n > 3072) the launch needs the opt-in
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(chol_upper_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    chol_upper_kernel<<<1, 1024, smem, st>>>(R, n);
     if (launches) *launches += 1;
     return cudaGetLastError();
 }

@@ -393,7 +393,7 @@ cudaError_t launch_si(const double* X, double* Q, int n, double tau2, int min_wa
 
 
 // =====================================================================================================================
-// Large embeddings (512 < n <= 2048): the same algorithm with the block kept in global memory (L2 resident) and the
+// Large embeddings (512 < n <= 4096): the same algorithm with the block kept in global memory (L2 resident) and the
 // Rayleigh-Ritz step done on the 32 x 32 projected matrix.  One step, given an orthonormal n x 32 basis Q:
 //   X = G Q (DMMA)            H = Q'X (32 x 32)            H = R Theta R'  (one-sided Jacobi, one CTA, registers)
 //   Q~ = Q R, X~ = X R        r_i = |x~_i - theta_i q~_i|  (Ritz pairs and residuals)

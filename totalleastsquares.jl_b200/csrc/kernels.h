@@ -41,9 +41,13 @@ cudaError_t launch_gram_reduce(const double* partial, int nsplit, int nblk, int 
 
 // TMA-fed SYRK for a materialised dense X (syrk_tma.cu): 128 x 128 blocks, 16-row boxes, 6-stage mbarrier ring
 constexpr int kSyrkBlk = 128;
-constexpr int kEigMaxN = 2048;              // largest min(M, N): 16 x 16 blocks of 128 columns
+constexpr int kEigMaxN = 4096;              // largest min(M, N): 32 x 32 blocks of 128 columns
 constexpr int kEigSmallN = 512;             // up to here: shared-memory / register-resident eigen kernels (eig.cu, eig_fast.cu)
-constexpr int kSyrkMaxBlk = 136;            // upper-triangular 128-blocks at N = 2048
+constexpr int kSyrkMaxBlk = 528;            // upper-triangular 128-blocks at N = 4096
+static_assert(kSyrkMaxBlk == (kEigMaxN / kSyrkBlk) * (kEigMaxN / kSyrkBlk + 1) / 2, "SyrkPlan tables cover kEigMaxN");
+// SyrkPlan is passed by value as a __grid_constant__ kernel parameter: 6392 bytes of parameters for syrk_reduce_kernel
+// and 6504 for syrk_tma_kernel (cuobjdump -elf, EIATTR_PARAM_CBANK).  That is above the 4 KB limit of toolkits before
+// CUDA 12.1 and within the 32 764 bytes that CUDA >= 12.1 allows on Volta and later.
 struct SyrkPlan {
     int nb, nblk, nsplit, ntiles, ncta;     // 128-blocks per dimension, upper-triangular blocks, -, 32-row tiles, CTAs
     int nsplit_blk[kSyrkMaxBlk];            // row splits (CTAs) of every block, proportional to its cost

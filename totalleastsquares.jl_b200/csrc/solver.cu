@@ -1055,7 +1055,7 @@ int rpca_cb_host(tlsq_handle* h, const double* Dh, int64_t M, int64_t N, const R
                  int64_t* sv_out, int64_t* iters_done, int32_t* converged, double* hist);
 
 // rpca_dev, continued on the dense device path (rpca_cb_host with its built-in hooks: full Jacobi SVT + exact stop test
-// every iteration, no rank limit) when a single-GPU solve leaves the accelerated kernels -- 512 < min(M,N) <= 2048 with
+// every iteration, no rank limit) when a single-GPU solve leaves the accelerated kernels -- 512 < min(M,N) <= 4096 with
 // a rank estimate above 32, or with hankel=true.  Slower, but the reference has no such limit either.
 int rpca_dev_any(tlsq_handle* h, const double* D, int64_t M, int64_t N, const RpcaParams& p, const RpcaOut& o) {
     t_dense_fallback = false;
@@ -1816,7 +1816,7 @@ int tlsq_rpca_f64(tlsq_handle* h, const double* D, int64_t M, int64_t N, double 
     t_dense_fallback = false;
     const int rc = rpca_dev(h, bD.as<double>(), M, N, p, o);
     if (rc == TLSQ_ERR_UNSUPPORTED && t_dense_fallback && h->nranks == 1) {
-        // 512 < min(M,N) <= 2048 with a rank estimate above 32, or with hankel=true: outside the factored kernels.  Repeat the solve on the
+        // 512 < min(M,N) <= 4096 with a rank estimate above 32, or with hankel=true: outside the factored kernels.  Repeat the solve on the
         // dense device path (full Jacobi SVT + exact stop test every iteration: the reference's loop statement by
         // statement, slower but without a rank limit) instead of failing.
         t_dense_fallback = false;
@@ -2023,6 +2023,21 @@ int tlsq_plan_fused_strips(uint8_t* tile_row, uint8_t* strip_col) {
 int tlsq_plan_hankel_shard(int64_t K, int nranks, int rank, int64_t* r0, int64_t* Kl) {
     if (K < 1 || nranks < 1 || rank < 0 || rank >= nranks || !r0 || !Kl) return set_err(TLSQ_ERR_ARG, "plan_hankel_shard: bad arguments");
     shard_hankel_rows(K, nranks, rank, r0, Kl);
+    return TLSQ_OK;
+}
+
+int tlsq_plan_syrk(int64_t M, int64_t N, int sm_count, int* nblk, int* ncta, int* nsplit_blk, int* cta_begin,
+                   int* part_off, int64_t* partial_bytes) {
+    if (M < 1 || N < 1 || sm_count < 1 || !nblk || !ncta || !nsplit_blk || !cta_begin || !part_off || !partial_bytes)
+        return set_err(TLSQ_ERR_ARG, "plan_syrk: bad arguments");
+    if (N > kEigMaxN) return set_err(TLSQ_ERR_UNSUPPORTED, "plan_syrk: N = %lld exceeds %d", (long long)N, kEigMaxN);
+    const SyrkPlan p = syrk_plan(M, N, sm_count);
+    *nblk = p.nblk;
+    *ncta = p.ncta;
+    memcpy(nsplit_blk, p.nsplit_blk, (size_t)p.nblk * sizeof(int));
+    memcpy(cta_begin, p.cta_begin, (size_t)(p.nblk + 1) * sizeof(int));
+    memcpy(part_off, p.part_off, (size_t)p.nblk * sizeof(int));
+    *partial_bytes = (int64_t)p.partial_bytes;
     return TLSQ_OK;
 }
 
