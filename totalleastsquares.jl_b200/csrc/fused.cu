@@ -130,22 +130,30 @@ struct FusedDev {
     int has_tp, has_tn, has_y, has_d;      // which TMA loads are issued per tile
 };
 
+// Rank pads above 16 exist for the implicit Hankel form only (kFusedMaxRankHankel).  Their layout differs in two places,
+// which brings RP = 32 to 229 712 B of shared memory:
+//   * no D tile: D comes from the signal through __ldg (has_d = 0), so Ys starts where Ds would (-32 KB);
+//   * Tsum keeps only the PEER's partial row sums; the own partial goes to Tps, whose T_{k-1} values have all been
+//     consumed by the A_{k-1} products before S1 and which is refilled by TMA only after C2 (-RP x 32 doubles).
+// The rank-r products run over 8-column chunks of the T rows, read from shared memory (see phases 2 and 4).
 template <int RP, bool HANKEL>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
 alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__ CUtensorMap mY,
                  const __grid_constant__ CUtensorMap mTp, const __grid_constant__ CUtensorMap mTn,
                  const __grid_constant__ CUtensorMap mYo, const __grid_constant__ CUtensorMap mTo, const FusedDev p) {
+    constexpr bool WIDE = RP > 16;
+    static_assert(!WIDE || (HANKEL && RP % 8 == 0 && RP <= kFusedMaxRankHankel), "rank pads above 16: Hankel form only");
     extern __shared__ __align__(1024) uint8_t smem[];
     double* W2s = reinterpret_cast<double*>(smem);              // [256][36] DMMA operand tile (both halves)
-    double* Ds = reinterpret_cast<double*>(smem + W2_BYTES);    // [128][32] own-half D tile          (TMA)
-    double* Ys = Ds + TILE_DOUBLES;                             // [128][32] own-half Y_{k-1} tile    (TMA)
+    double* Ds = reinterpret_cast<double*>(smem + W2_BYTES);    // [128][32] own-half D tile          (TMA; absent if WIDE)
+    double* Ys = Ds + (WIDE ? 0 : TILE_DOUBLES);                // [128][32] own-half Y_{k-1} tile    (TMA)
     double* Es = Ys + TILE_DOUBLES;                             // [128][32] E_k (or the Gram operand in W / D mode)
     double* Vps = Es + TILE_DOUBLES;                            // [128][RP] own-half rows of V_{k-1}
     double* Vks = Vps + FH * RP;                                // [128][RP] own-half rows of V_k
     double* Tps = Vks + FH * RP;                                // [RP][32]  T_{k-1} tile             (TMA)
     double* Tns = Tps + RP * FR;                                // [RP][32]  T_k tile: TMA load when given, else TMA-store staging
-    double* Tsum = Tns + RP * FR;                               // [2][RP][32] partial row sums of the two CTAs
-    double* fs = Tsum + 2 * RP * FR;                            // [RP] shrink factors
+    double* Tsum = Tns + RP * FR;                               // [2][RP][32] partial row sums of the two CTAs (WIDE: [RP][32], the peer's)
+    double* fs = Tsum + (WIDE ? 1 : 2) * RP * FR;               // [RP] shrink factors
     double* red = fs + RP;                                      // [8]
     uint64_t* bar = reinterpret_cast<uint64_t*>(red + 8);
     double* Tpart = W2s;                                        // [8][RP][32] aliases the operand tile (see S3)
@@ -228,6 +236,68 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
                 const double d = HANKEL ? (rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0) : Ds[jl * FR + lane];
                 Es[jl * FR + lane] = d;
             }
+        } else if constexpr (WIDE) {
+            // A_{k-1} over all 16 columns of the warp at once (16 independent FMA chains), the T_{k-1} row taken from
+            // shared memory 8 columns at a time: 16 + 8 registers next to the accumulators instead of 2 RP
+            double av[16], wv[16];
+#pragma unroll
+            for (int u = 0; u < 16; ++u) av[u] = 0.0;
+#pragma unroll 1
+            for (int h = 0; h < RP; h += 8) {
+                double tc[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) tc[j] = (p.has_tp && h + j < a.svp_prev) ? Tps[(h + j) * FR + lane] : 0.0;
+#pragma unroll
+                for (int u = 0; u < 16; ++u) {
+                    const double* v = Vps + (16 * warp + u) * RP + h;
+#pragma unroll
+                    for (int j = 0; j < 8; j += 2) {
+                        const double2 vv = *reinterpret_cast<const double2*>(v + j);
+                        av[u] = fma(tc[j], vv.x, av[u]);
+                        av[u] = fma(tc[j + 1], vv.y, av[u]);
+                    }
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < 16; ++u) {
+                const int jl = 16 * warp + u;
+                const double d = rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0;
+                const double yp = Ys[jl * FR + lane];
+                const double ap = (nnA && !(__double_as_longlong(av[u]) > 0)) ? 0.0 : av[u];
+                double e, w;
+                alm_ew(d, ap, yp, a.im, a.eps, a.nonnegE, e, w);
+                Es[jl * FR + lane] = (go == FUSED_GRAM_W) ? w : e;
+                wv[u] = w;
+            }
+            if (a.compute_T) {
+                // partial row sums of T = W_k V_k, 8 columns at a time (u ascending per column, as below)
+#pragma unroll 1
+                for (int h = 0; h < RP; h += 8) {
+                    double tr[8];
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) tr[j] = 0.0;
+#pragma unroll
+                    for (int u = 0; u < 16; ++u) {
+                        const double* v = Vks + (16 * warp + u) * RP + h;
+#pragma unroll
+                        for (int j = 0; j < 8; j += 2) {
+                            const double2 vv = *reinterpret_cast<const double2*>(v + j);
+                            tr[j] = fma(wv[u], vv.x, tr[j]);
+                            tr[j + 1] = fma(wv[u], vv.y, tr[j + 1]);
+                        }
+                    }
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) Tpart[(warp * RP + h + j) * FR + lane] = tr[j];
+                }
+                __syncthreads();                                                       // S1: Tps is consumed
+                for (int idx = tid; idx < RP * FR; idx += 256) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int w8 = 0; w8 < 8; ++w8) s += Tpart[w8 * RP * FR + idx];
+                    Tps[idx] = s;                                                      // own partial
+                    st_cluster(tsum_peer + (uint32_t)(idx * 8), s);                    // the peer's Tsum
+                }
+            }
         } else {
             // staged in batches of UB elements so that every stage exposes UB independent dependency chains (the
             // FP64 pipe is shared by only two warps per scheduler: instruction-level parallelism must hide its latency)
@@ -288,6 +358,52 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
             for (int u = 0; u < 16; ++u) {
                 const int jl = 16 * warp + u;
                 const double val = Es[jl * FR + lane];
+                const int off = (c0 + jl) * FWS + lane;
+                W2s[off] = val;
+                if (push) st_cluster(w2_peer + (uint32_t)off * 8u, val);
+            }
+        } else if constexpr (WIDE) {
+            // A_k over the warp's 16 columns, the T_k row formed (or read) 8 columns at a time; own + peer partial is
+            // the same sum as Tsum[0] + Tsum[1] on either CTA (FP64 addition commutes)
+            double av[16];
+#pragma unroll
+            for (int u = 0; u < 16; ++u) av[u] = 0.0;
+#pragma unroll 1
+            for (int h = 0; h < RP; h += 8) {
+                double tc[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const int c = h + j;
+                    tc[j] = a.compute_T ? fs[c] * (Tps[c * FR + lane] + Tsum[c * FR + lane])
+                                        : (c < a.svp ? Tns[c * FR + lane] : 0.0);
+                }
+#pragma unroll
+                for (int u = 0; u < 16; ++u) {
+                    const double* v = Vks + (16 * warp + u) * RP + h;
+#pragma unroll
+                    for (int j = 0; j < 8; j += 2) {
+                        const double2 vv = *reinterpret_cast<const double2*>(v + j);
+                        av[u] = fma(tc[j], vv.x, av[u]);
+                        av[u] = fma(tc[j + 1], vv.y, av[u]);
+                    }
+                }
+            }
+            if (a.compute_T && rank == 0)                                              // staged for the TMA store
+                for (int c = warp; c < RP; c += 8) Tns[c * FR + lane] = fs[c] * (Tps[c * FR + lane] + Tsum[c * FR + lane]);
+#pragma unroll
+            for (int u = 0; u < 16; ++u) {
+                const int jl = 16 * warp + u;
+                const double d = rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0;
+                const double yp = Ys[jl * FR + lane];
+                const double e = Es[jl * FR + lane];
+                const double an = (nnA && !(__double_as_longlong(av[u]) > 0)) ? 0.0 : av[u];   // max.(A, 0) :218
+                const double z = __dsub_rn(__dsub_rn(d, an), e);                    // @. Z = D - A - E  :221
+                const double yn = __dadd_rn(yp, __dmul_rn(a.mu, z));                // @. Y = Y + mu*Z   :222
+                zz = fma(z, z, zz);
+                Es[jl * FR + lane] = yn;                                            // staged for the TMA store
+                double e2, w2;
+                alm_ew(d, an, yn, a.im_next, a.eps_next, a.nonnegE, e2, w2);        // SVT input of iteration k+1
+                const double val = (go == FUSED_GRAM_WNEXT) ? w2 : z;
                 const int off = (c0 + jl) * FWS + lane;
                 W2s[off] = val;
                 if (push) st_cluster(w2_peer + (uint32_t)off * 8u, val);
@@ -464,11 +580,14 @@ FusedStripTab make_tab() {
     return tb;
 }
 
+// RP = 16: 221 392 B; RP = 24 (Hankel): 207 120 B; RP = 32 (Hankel): 229 712 B -- all within the 232 448 B of a block
 template <int RP>
-size_t smem_bytes() {
-    return (size_t)W2_BYTES + 3 * (size_t)TILE_BYTES + 2 * (size_t)FH * RP * 8 + 2 * (size_t)RP * FR * 8 +
-           2 * (size_t)RP * FR * 8 + (size_t)RP * 8 + 8 * 8 + 16;
+constexpr size_t smem_bytes() {
+    constexpr bool wide = RP > 16;          // no D tile, one Tsum half (see alm_fused_kernel)
+    return (size_t)W2_BYTES + (wide ? 2 : 3) * (size_t)TILE_BYTES + 2 * (size_t)FH * RP * 8 + 2 * (size_t)RP * FR * 8 +
+           (wide ? 1 : 2) * (size_t)RP * FR * 8 + (size_t)RP * 8 + 8 * 8 + 16;
 }
+static_assert(smem_bytes<kFusedMaxRankHankel>() <= 232448, "one-pass kernel: shared memory of a block");
 
 struct Inst {
     int ncluster = -1;      // co-resident clusters (queried once)
@@ -532,8 +651,12 @@ bool fused_eligible(const MatSrc& D, bool hankel, int64_t M, int64_t N) {
     return encode_fn() != nullptr;
 }
 
+int fused_max_rank(bool hankel) { return hankel ? kFusedMaxRankHankel : kFusedMaxRankDense; }
+
+// 4, 8, 12, 16, then 24 and 32 (Hankel form only)
 int fused_rank_pad(int svp, int svp_prev) {
     const int m = svp > svp_prev ? svp : svp_prev;
+    if (m > 16) return m <= 24 ? 24 : 32;
     return m <= 4 ? 4 : ((m + 3) & ~3);
 }
 
@@ -542,7 +665,7 @@ cudaError_t launch_alm_fused(const FusedArgs& a, bool hankel, const double* Yp, 
     static const FusedStripTab tab = make_tab();
     if (!encode_fn()) return cudaErrorNotSupported;
     const int rp = fused_rank_pad(a.svp, a.svp_prev);
-    if (rp > kFusedMaxRank) return cudaErrorInvalidValue;
+    if (rp > fused_max_rank(hankel)) return cudaErrorInvalidValue;
     FusedDev p = {};
     p.a = a;
     p.tab = tab;
@@ -575,7 +698,9 @@ cudaError_t launch_alm_fused(const FusedArgs& a, bool hankel, const double* Yp, 
         case 4:  e = launch_rp<4>(hankel, m, p, sm_count, st, &nc); break;
         case 8:  e = launch_rp<8>(hankel, m, p, sm_count, st, &nc); break;
         case 12: e = launch_rp<12>(hankel, m, p, sm_count, st, &nc); break;
-        default: e = launch_rp<16>(hankel, m, p, sm_count, st, &nc); break;
+        case 16: e = launch_rp<16>(hankel, m, p, sm_count, st, &nc); break;
+        case 24: e = launch_inst<24, true>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, &nc); break;
+        default: e = launch_inst<32, true>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, &nc); break;
     }
     if (e != cudaSuccess) return e;
     fused_reduce_kernel<<<(FN * FN + 255) / 256, 256, 0, st>>>(a.partial, nc, a.zpart, 2 * nc, G, zz_out);

@@ -211,7 +211,12 @@ cudaError_t launch_z_from_factors(const EpiArgs& a, bool hankel, int svp, double
 // kernel (thread-block cluster pair per 32-row tile, DSMEM exchange, TMA staging, DMMA Gram).  W is never materialised.
 // ----------------------------------------------------------------------------------------------------
 constexpr int kFusedN = 256;
-constexpr int kFusedMaxRank = 16;
+// largest rank estimate of the one-pass kernel: rank pads 4..16 for dense D, and also 24 and 32 for the implicit Hankel
+// form (whose instances free the D tile for the wider V / T blocks); above the cap the solver hands over to the
+// streaming pipeline
+constexpr int kFusedMaxRankDense = 16;
+constexpr int kFusedMaxRankHankel = 32;
+static_assert(kFusedMaxRankHankel <= kStreamMaxRank, "the one-pass kernel reads T from the M x 32 factor");
 enum FusedGram : int {
     FUSED_GRAM_WNEXT = 0,   // operand = W_{k+1} = (D - E_{k+1}) + Y_k/mu_{k+1}          (the normal step)
     FUSED_GRAM_Z = 1,       // operand = Z_k = (D - A_k) - E_k                            (exact stop test, :225)
@@ -240,6 +245,7 @@ struct FusedArgs {
 size_t fused_partial_doubles(int sm_count);
 FusedStripTab fused_strip_table();      // which 32 x 8 Gram strips every (CTA of the pair, warp) accumulates
 bool fused_eligible(const MatSrc& D, bool hankel, int64_t M, int64_t N);
+int fused_max_rank(bool hankel);
 int fused_rank_pad(int svp, int svp_prev);
 // G (256 x 256) = Gram of the chosen operand; zz_out (nullable) = ||Z_k||_F^2
 cudaError_t launch_alm_fused(const FusedArgs& a, bool hankel, const double* Yp, const double* Tp, const double* Tn_given,

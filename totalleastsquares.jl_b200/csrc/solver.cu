@@ -622,11 +622,13 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
             if (inplace_y && no_pred && !exact_cost) want_z = false;
             if (inplace_y && k >= two_phase_from) want_z = true;
         }
-        if (fused && (svp > kFusedMaxRank || svpb[cur] > kFusedMaxRank)) {
+        const int fused_cap = fused_max_rank(hankel);      // 16 for dense D, 32 for the implicit Hankel form
+        if (fused && (svp > fused_cap || svpb[cur] > fused_cap)) {
             // rank estimate beyond the fused kernel: materialise W_k once and continue on the streaming pipeline
             if (ldp != M || inplace_y || !all_legacy)
-                return set_err(TLSQ_ERR_UNSUPPORTED, "rpca: rank estimate %d exceeds the one-pass kernel's %d and the "
-                               "streaming pipeline cannot take over (padded / in-place dual variable)", svp, kFusedMaxRank);
+                return set_err(TLSQ_ERR_UNSUPPORTED, "rpca: rank estimate %d exceeds the one-pass kernel's cap of %d "
+                               "(%s) and the streaming pipeline cannot take over (padded / in-place dual variable)", svp,
+                               fused_cap, hankel ? "implicit Hankel" : "dense D");
             CK(ensure_w());
             EpiArgs wa = {};
             wa.D = D; wa.Yp = Ybuf[cur]; wa.Tp = Tb[cur]; wa.Vp = Vb[cur]; wa.svp_prev = svpb[cur];

@@ -54,6 +54,19 @@ def sinusoid_np(Ns: int, seed: int = 5, miss_frac: float = 0.1, noise: float = 0
     return y, yn
 
 
+def sinusoids_np(Ns: int, k: int, seed: int = 5, noise: float = 0.05, outlier_frac: float = 0.01):
+    """Sum of k sinusoids (frequencies in [0.02, 0.92), random phases, amplitudes in [0.5, 1.5)), `noise` N(0,1) noise
+    and `outlier_frac` of the samples shifted by +5.  The Hankel rank of the clean signal is 2k, so the rank estimate
+    of lowrankfilter grows with k.  Returns (clean, noisy)."""
+    rng = np.random.default_rng(seed)
+    t = np.arange(Ns)
+    freqs = 0.02 + 0.9 * rng.random(k)
+    y0 = sum(np.sin(f * t + rng.random() * 6.28) * (0.5 + rng.random()) for f in freqs)
+    y = y0 + noise * rng.standard_normal(Ns)
+    y[rng.random(Ns) < outlier_frac] += 5.0
+    return y0, y
+
+
 def lowrank_sparse_cuda(r0: int, r1: int, N: int, device, r: int = 10, frac: float = 0.05, seed: int = 4,
                         nonneg: bool = True):
     """Rows [r0, r1) of the global low-rank + sparse matrix as a column-major CUDA tensor (shape (r1-r0, N)).
