@@ -155,15 +155,21 @@ unhankel_divide_kernel(const double* __restrict__ sum, const double* __restrict_
     }
 }
 
-// Anti-diagonal sums of A = clamp(T V') over the local Hankel rows [r0, r0 + Kl), lag 1, WITHOUT materialising A
-// (unhankel of src/robustPCA.jl:28-39 applied to the factored iterate):
-//   sum[k] = sum_{j} clamp(T[k - j - r0, :] . V[j, :]),   0 <= k - j - r0 < Kl
-// A block owns 256 consecutive samples k; the 256 + n - 1 rows of T it needs are staged in shared memory.
+// Sums of A = clamp(T V') over {(k, j): k lag + j = t} for the local Hankel rows k in [r0, r0 + Kl), WITHOUT
+// materialising A (unhankel of src/robustPCA.jl:53-68 applied to the factored iterate; lag 1 is :28-39):
+//   sum[t] = sum_{j = t mod lag, step lag} clamp(T[(t - j) / lag - r0, :] . V[j, :]),   0 <= (t - j) / lag - r0 < Kl
+// Terms are added for increasing j (decreasing k), the order of unhankel_kernel, so the sums are those of the dense
+// route bit for bit.  A block owns 256 consecutive samples t; the rows k with 0 <= t - k lag < n for some of them,
+// k in [ceil((t0 - n + 1) / lag), floor((t0 + 255) / lag)], at most (254 + n) / lag + 1, are staged in shared memory.
+__device__ __forceinline__ int64_t ceil_div_any(int64_t a, int64_t b) {        // b > 0, a of either sign
+    return a >= 0 ? (a + b - 1) / b : -((-a) / b);
+}
+
 __global__ void __launch_bounds__(256)
 unhankel_factors_kernel(const double* __restrict__ T, int64_t ldt, const double* __restrict__ V, int rp, int nonnegA,
-                        int64_t r0, int64_t Kl, int n, int64_t Ns, double* __restrict__ sum) {
+                        int64_t r0, int64_t Kl, int n, int lag, int64_t Ns, double* __restrict__ sum) {
     extern __shared__ double sm[];
-    const int span = 256 + n - 1;
+    const int span = (254 + n) / lag + 1;
     double* Vsm = sm;                        // [n][rp]
     double* Tsm = sm + (size_t)n * rp;       // [rp][span]
     for (int idx = threadIdx.x; idx < n * rp; idx += 256) {
@@ -172,8 +178,9 @@ unhankel_factors_kernel(const double* __restrict__ T, int64_t ldt, const double*
     }
     const int64_t nblk = (Ns + 255) / 256;
     for (int64_t b = blockIdx.x; b < nblk; b += gridDim.x) {
-        const int64_t kb = b * 256;
-        const int64_t ilo = kb - r0 - (n - 1);
+        const int64_t tb = b * 256;
+        const int64_t klo = ceil_div_any(tb - (n - 1), lag);      // first staged Hankel row
+        const int64_t ilo = klo - r0;
         __syncthreads();
         for (int idx = threadIdx.x; idx < rp * span; idx += 256) {
             const int q = idx % span, c = idx / span;
@@ -181,11 +188,12 @@ unhankel_factors_kernel(const double* __restrict__ T, int64_t ldt, const double*
             Tsm[c * span + q] = (i >= 0 && i < Kl) ? __ldg(T + (int64_t)c * ldt + i) : 0.0;
         }
         __syncthreads();
-        const int64_t k = kb + threadIdx.x;
-        if (k < Ns) {
+        const int64_t t = tb + threadIdx.x;
+        if (t < Ns) {
             double s = 0.0;
-            for (int j = 0; j < n; ++j) {
-                const int q = (int)threadIdx.x + (n - 1) - j;
+            const int j0 = (int)((tb % lag + threadIdx.x) % lag);
+            int q = (int)((t - j0) / lag - klo);                   // staged row of (t, j): one less per step of j
+            for (int j = j0; j < n; j += lag, --q) {
                 const int64_t i = ilo + q;
                 if (i < 0 || i >= Kl) continue;
                 double av = 0.0;
@@ -193,7 +201,7 @@ unhankel_factors_kernel(const double* __restrict__ T, int64_t ldt, const double*
                 if (nonnegA) av = (__double_as_longlong(av) > 0) ? av : 0.0;
                 s += av;
             }
-            sum[k] = s;
+            sum[t] = s;
         }
     }
 }
@@ -202,31 +210,35 @@ unhankel_factors_kernel(const double* __restrict__ T, int64_t ldt, const double*
 // not fit in shared memory (n > 256 with a large rank estimate).  Once per solve, latency is irrelevant.
 __global__ void __launch_bounds__(256)
 unhankel_factors_direct_kernel(const double* __restrict__ T, int64_t ldt, const double* __restrict__ V, int rp,
-                               int nonnegA, int64_t r0, int64_t Kl, int n, int64_t Ns, double* __restrict__ sum) {
-    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < Ns; k += (int64_t)gridDim.x * blockDim.x) {
+                               int nonnegA, int64_t r0, int64_t Kl, int n, int lag, int64_t Ns,
+                               double* __restrict__ sum) {
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < Ns; t += (int64_t)gridDim.x * blockDim.x) {
         double s = 0.0;
-        for (int j = 0; j < n; ++j) {
-            const int64_t i = k - r0 - j;
+        const int j0 = (int)(t % lag);
+        int64_t i = (t - j0) / lag - r0;                          // local row of (t, j): one less per step of j
+        for (int j = j0; j < n; j += lag, --i) {
             if (i < 0 || i >= Kl) continue;
             double av = 0.0;
             for (int c = 0; c < rp; ++c) av = fma(__ldg(T + (int64_t)c * ldt + i), __ldg(V + (int64_t)c * n + j), av);
             if (nonnegA) av = (__double_as_longlong(av) > 0) ? av : 0.0;
             s += av;
         }
-        sum[k] = s;
+        sum[t] = s;
     }
 }
 
-// y[k] = sum[k] / #{(i, j): i + j = k, 0 <= i < K, 0 <= j < n}   (lag 1; the count is known in closed form)
+// y[t] = sum[t] / max(#{k in [0, K): 0 <= t - k lag < n}, 1)   (:66; the count is known in closed form: k runs from
+// max(0, ceil((t - n + 1) / lag)) to min(K - 1, floor(t / lag)).  Samples no row covers -- the last (Ns - n) % lag --
+// have sum 0 and get 0.)
 __global__ void __launch_bounds__(256)
-unhankel_divide_count_kernel(const double* __restrict__ sum, int64_t K, int64_t n, int64_t Ns, double* __restrict__ y) {
-    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < Ns; k += (int64_t)gridDim.x * blockDim.x) {
-        int64_t c = k;
-        if (n - 1 < c) c = n - 1;
-        if (K - 1 < c) c = K - 1;
-        if (K + n - 2 - k < c) c = K + n - 2 - k;
-        c = c < 0 ? 1 : c + 1;
-        y[k] = sum[k] / (double)c;
+unhankel_divide_count_kernel(const double* __restrict__ sum, int64_t K, int64_t n, int64_t lag, int64_t Ns,
+                             double* __restrict__ y) {
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < Ns; t += (int64_t)gridDim.x * blockDim.x) {
+        int64_t lo = lag == 1 ? t - n + 1 : ceil_div_any(t - n + 1, lag), hi = lag == 1 ? t : t / lag;
+        if (lo < 0) lo = 0;
+        if (hi > K - 1) hi = K - 1;
+        const int64_t c = hi >= lo ? hi - lo + 1 : 1;
+        y[t] = sum[t] / (double)c;
     }
 }
 
@@ -432,15 +444,16 @@ cudaError_t launch_unhankel_divide(const double* sum, const double* cnt, int64_t
 }
 
 cudaError_t launch_unhankel_factors(const double* T, int64_t ldt, const double* V, int svp, int nonnegA, int64_t r0,
-                                    int64_t Kl, int64_t n, int64_t Ns, double* sum, int sm_count, cudaStream_t st,
-                                    int64_t* launches) {
+                                    int64_t Kl, int64_t n, int64_t lag, int64_t Ns, double* sum, int sm_count,
+                                    cudaStream_t st, int64_t* launches) {
     if (svp < 1) return cudaMemsetAsync(sum, 0, (size_t)Ns * sizeof(double), st);     // A = 0
     const int rp = svp;
-    const size_t smem = ((size_t)n * rp + (size_t)rp * (256 + n - 1)) * sizeof(double);
+    const size_t smem = ((size_t)n * rp + (size_t)rp * ((254 + n) / lag + 1)) * sizeof(double);
     if (smem > (size_t)220 * 1024) {
         int64_t blocks = (Ns + 255) / 256;
         if (blocks > (int64_t)sm_count * 8) blocks = (int64_t)sm_count * 8;
-        unhankel_factors_direct_kernel<<<(unsigned)blocks, 256, 0, st>>>(T, ldt, V, rp, nonnegA, r0, Kl, (int)n, Ns, sum);
+        unhankel_factors_direct_kernel<<<(unsigned)blocks, 256, 0, st>>>(T, ldt, V, rp, nonnegA, r0, Kl, (int)n, (int)lag,
+                                                                          Ns, sum);
         if (launches) *launches += 1;
         return cudaGetLastError();
     }
@@ -449,14 +462,15 @@ cudaError_t launch_unhankel_factors(const double* T, int64_t ldt, const double* 
     if (e != cudaSuccess) return e;
     int64_t blocks = (Ns + 255) / 256;
     if (blocks > (int64_t)sm_count * 4) blocks = (int64_t)sm_count * 4;
-    unhankel_factors_kernel<<<(unsigned)blocks, 256, smem, st>>>(T, ldt, V, rp, nonnegA, r0, Kl, (int)n, Ns, sum);
+    unhankel_factors_kernel<<<(unsigned)blocks, 256, smem, st>>>(T, ldt, V, rp, nonnegA, r0, Kl, (int)n, (int)lag, Ns,
+                                                                 sum);
     if (launches) *launches += 1;
     return cudaGetLastError();
 }
 
-cudaError_t launch_unhankel_divide_count(const double* sum, int64_t K, int64_t n, int64_t Ns, double* y, cudaStream_t st,
-                                         int64_t* launches) {
-    unhankel_divide_count_kernel<<<stream_grid(Ns, 148), 256, 0, st>>>(sum, K, n, Ns, y);
+cudaError_t launch_unhankel_divide_count(const double* sum, int64_t K, int64_t n, int64_t lag, int64_t Ns, double* y,
+                                         cudaStream_t st, int64_t* launches) {
+    unhankel_divide_count_kernel<<<stream_grid(Ns, 148), 256, 0, st>>>(sum, K, n, lag, Ns, y);
     if (launches) *launches += 1;
     return cudaGetLastError();
 }

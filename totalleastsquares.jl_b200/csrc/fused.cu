@@ -136,13 +136,16 @@ struct FusedDev {
 //   * Tsum keeps only the PEER's partial row sums; the own partial goes to Tps, whose T_{k-1} values have all been
 //     consumed by the A_{k-1} products before S1 and which is refilled by TMA only after C2 (-RP x 32 doubles).
 // The rank-r products run over 8-column chunks of the T rows, read from shared memory (see phases 2 and 4).
-template <int RP, bool HANKEL>
+// LAG (Hankel form only): D[row, c] = y[row * lag + c] with the lag a runtime value.  The lag-1 instances keep the
+// address y + row + c: a runtime lag there costs registers that the RP >= 8 instances pay for in new spills.
+template <int RP, bool HANKEL, bool LAG>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
 alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__ CUtensorMap mY,
                  const __grid_constant__ CUtensorMap mTp, const __grid_constant__ CUtensorMap mTn,
                  const __grid_constant__ CUtensorMap mYo, const __grid_constant__ CUtensorMap mTo, const FusedDev p) {
     constexpr bool WIDE = RP > 16;
     static_assert(!WIDE || (HANKEL && RP % 8 == 0 && RP <= kFusedMaxRankHankel), "rank pads above 16: Hankel form only");
+    static_assert(HANKEL || !LAG, "a lag exists for the Hankel form only");
     extern __shared__ __align__(1024) uint8_t smem[];
     double* W2s = reinterpret_cast<double*>(smem);              // [256][36] DMMA operand tile (both halves)
     double* Ds = reinterpret_cast<double*>(smem + W2_BYTES);    // [128][32] own-half D tile          (TMA; absent if WIDE)
@@ -226,6 +229,10 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
     for (int tile = cl; tile < p.ntiles; tile += p.ncluster, ++it) {
         const int64_t row = (int64_t)tile * FR + lane;
         const bool rowok = row < a.M;
+        // Hankel form: D[row, c0 + jl] = y[row * lag + c0 + jl] (read only when rowok); with LAG the row's base is formed
+        // once per tile, lag 1 keeps its original address expression
+        const double* drow = a.D.p + (LAG && rowok ? row * a.D.ld : 0) + c0;
+        auto hk_d = [&](int jl) -> double { return LAG ? __ldg(drow + jl) : __ldg(a.D.p + row + c0 + jl); };
         mbar_wait(bar, (uint32_t)(it & 1));
 
         // ---- phase 2: E_k, W_k and the partial row sums of T = W_k V_k over this warp's 16 columns --------------
@@ -233,7 +240,7 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
 #pragma unroll 1
             for (int u = 0; u < 16; ++u) {
                 const int jl = 16 * warp + u;
-                const double d = HANKEL ? (rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0) : Ds[jl * FR + lane];
+                const double d = HANKEL ? (rowok ? hk_d(jl) : 0.0) : Ds[jl * FR + lane];
                 Es[jl * FR + lane] = d;
             }
         } else if constexpr (WIDE) {
@@ -261,7 +268,7 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
 #pragma unroll
             for (int u = 0; u < 16; ++u) {
                 const int jl = 16 * warp + u;
-                const double d = rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0;
+                const double d = rowok ? hk_d(jl) : 0.0;
                 const double yp = Ys[jl * FR + lane];
                 const double ap = (nnA && !(__double_as_longlong(av[u]) > 0)) ? 0.0 : av[u];
                 double e, w;
@@ -315,7 +322,7 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
 #pragma unroll
                 for (int u = 0; u < UB; ++u) {
                     const int jl = 16 * warp + u0 + u;
-                    const double d = HANKEL ? (rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0) : Ds[jl * FR + lane];
+                    const double d = HANKEL ? (rowok ? hk_d(jl) : 0.0) : Ds[jl * FR + lane];
                     const double yp = Ys[jl * FR + lane];
                     const double ap = (nnA && !(__double_as_longlong(av[u]) > 0)) ? 0.0 : av[u];
                     double e, w;
@@ -393,7 +400,7 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
 #pragma unroll
             for (int u = 0; u < 16; ++u) {
                 const int jl = 16 * warp + u;
-                const double d = rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0;
+                const double d = rowok ? hk_d(jl) : 0.0;
                 const double yp = Ys[jl * FR + lane];
                 const double e = Es[jl * FR + lane];
                 const double an = (nnA && !(__double_as_longlong(av[u]) > 0)) ? 0.0 : av[u];   // max.(A, 0) :218
@@ -428,7 +435,7 @@ alm_fused_kernel(const __grid_constant__ CUtensorMap mD, const __grid_constant__
 #pragma unroll
                 for (int u = 0; u < UB; ++u) {
                     const int jl = 16 * warp + u0 + u;
-                    const double d = HANKEL ? (rowok ? __ldg(a.D.p + row + c0 + jl) : 0.0) : Ds[jl * FR + lane];
+                    const double d = HANKEL ? (rowok ? hk_d(jl) : 0.0) : Ds[jl * FR + lane];
                     const double yp = Ys[jl * FR + lane];
                     const double e = Es[jl * FR + lane];
                     const double an = (nnA && !(__double_as_longlong(av[u]) > 0)) ? 0.0 : av[u];   // max.(A, 0) :218
@@ -610,12 +617,12 @@ int query_clusters(Kern kern, int threads, size_t smem, int sm_count) {
     return nc < 1 ? 1 : nc;
 }
 
-template <int RP, bool HANKEL>
+template <int RP, bool HANKEL, bool LAG>
 cudaError_t launch_inst(const CUtensorMap& mD, const CUtensorMap& mY, const CUtensorMap& mTp, const CUtensorMap& mTn,
                         const CUtensorMap& mYo, const CUtensorMap& mTo, FusedDev p, int sm_count, cudaStream_t st,
                         int* ncluster_out) {
     static Inst inst;
-    auto kern = alm_fused_kernel<RP, HANKEL>;
+    auto kern = alm_fused_kernel<RP, HANKEL, LAG>;
     const size_t smem = smem_bytes<RP>();
     if (inst.ncluster < 0) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -630,10 +637,15 @@ cudaError_t launch_inst(const CUtensorMap& mD, const CUtensorMap& mY, const CUte
     return cudaGetLastError();
 }
 
+// Hankel forms for every rank pad; the dense form only up to kFusedMaxRankDense
 template <int RP>
-cudaError_t launch_rp(bool hankel, const CUtensorMap* m, const FusedDev& p, int sm_count, cudaStream_t st, int* nc) {
-    return hankel ? launch_inst<RP, true>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, nc)
-                  : launch_inst<RP, false>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, nc);
+cudaError_t launch_rp(bool hankel, bool lag, const CUtensorMap* m, const FusedDev& p, int sm_count, cudaStream_t st,
+                      int* nc) {
+    if (hankel && lag) return launch_inst<RP, true, true>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, nc);
+    if (hankel) return launch_inst<RP, true, false>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, nc);
+    if constexpr (RP <= kFusedMaxRankDense)
+        return launch_inst<RP, false, false>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, nc);
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace
@@ -646,7 +658,7 @@ size_t fused_partial_doubles(int sm_count) {
 
 bool fused_eligible(const MatSrc& D, bool hankel, int64_t M, int64_t N) {
     if (N != FN || M < 4096 || M >= ((int64_t)1 << 31)) return false;
-    if (hankel) { if (D.ld != 1) return false; }        // Y / T live in padded (even) leading dimensions: any M
+    if (hankel) { if (D.ld < 1) return false; }         // any lag; Y / T live in padded (even) leading dimensions: any M
     else if ((M & 1) || (D.ld & 1) || (reinterpret_cast<uintptr_t>(D.p) & 15)) return false;
     return encode_fn() != nullptr;
 }
@@ -693,14 +705,15 @@ cudaError_t launch_alm_fused(const FusedArgs& a, bool hankel, const double* Yp, 
     if (needs_tk && a.write_Y && !a.Yn) return cudaErrorInvalidValue;
     p.a.VpT = nullptr;
     int nc = 0;
+    const bool lagged = hankel && a.D.ld != 1;
     cudaError_t e;
     switch (rp) {
-        case 4:  e = launch_rp<4>(hankel, m, p, sm_count, st, &nc); break;
-        case 8:  e = launch_rp<8>(hankel, m, p, sm_count, st, &nc); break;
-        case 12: e = launch_rp<12>(hankel, m, p, sm_count, st, &nc); break;
-        case 16: e = launch_rp<16>(hankel, m, p, sm_count, st, &nc); break;
-        case 24: e = launch_inst<24, true>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, &nc); break;
-        default: e = launch_inst<32, true>(m[0], m[1], m[2], m[3], m[4], m[5], p, sm_count, st, &nc); break;
+        case 4:  e = launch_rp<4>(hankel, lagged, m, p, sm_count, st, &nc); break;
+        case 8:  e = launch_rp<8>(hankel, lagged, m, p, sm_count, st, &nc); break;
+        case 12: e = launch_rp<12>(hankel, lagged, m, p, sm_count, st, &nc); break;
+        case 16: e = launch_rp<16>(hankel, lagged, m, p, sm_count, st, &nc); break;
+        case 24: e = launch_rp<24>(hankel, lagged, m, p, sm_count, st, &nc); break;
+        default: e = launch_rp<32>(hankel, lagged, m, p, sm_count, st, &nc); break;
     }
     if (e != cudaSuccess) return e;
     fused_reduce_kernel<<<(FN * FN + 255) / 256, 256, 0, st>>>(a.partial, nc, a.zpart, 2 * nc, G, zz_out);

@@ -225,7 +225,7 @@ enum FusedGram : int {
 };
 struct FusedStripTab { uint8_t row[2][8][9]; uint8_t cs[2][8][9]; };
 struct FusedArgs {
-    MatSrc D;               // dense (TMA) or implicit Hankel signal with lag 1
+    MatSrc D;               // dense (TMA) or implicit Hankel signal (any lag: D[row, c] = y[row * lag + c])
     const double* Vp;       // V_{k-1}: 256 x >= svp_prev (ld 256)
     const double* Vs;       // V_k:     256 x >= svp      (ld 256)
     const double* fvec;     // shrink factors of iteration k
@@ -302,13 +302,13 @@ cudaError_t launch_unhankel_partial(const double* A, int64_t r0, int64_t Kl, int
 cudaError_t launch_unhankel_divide(const double* sum, const double* cnt, int64_t Ns, double* y, cudaStream_t st,
                                    int64_t* launches);
 
-// unhankel of the FACTORED iterate A = clamp(T V') (lag 1): sum[k] over the local Hankel rows [r0, r0+Kl); every k in
-// [0, Ns) is written (0 where this shard does not contribute); the count is closed-form (divide_count)
+// unhankel of the FACTORED iterate A = clamp(T V') (any lag <= n): sum[t] over the local Hankel rows [r0, r0+Kl); every
+// t in [0, Ns) is written (0 where this shard does not contribute); the count is closed-form (divide_count)
 cudaError_t launch_unhankel_factors(const double* T, int64_t ldt, const double* V, int svp, int nonnegA, int64_t r0,
-                                    int64_t Kl, int64_t n, int64_t Ns, double* sum, int sm_count, cudaStream_t st,
-                                    int64_t* launches);
-cudaError_t launch_unhankel_divide_count(const double* sum, int64_t K, int64_t n, int64_t Ns, double* y, cudaStream_t st,
-                                         int64_t* launches);
+                                    int64_t Kl, int64_t n, int64_t lag, int64_t Ns, double* sum, int sm_count,
+                                    cudaStream_t st, int64_t* launches);
+cudaError_t launch_unhankel_divide_count(const double* sum, int64_t K, int64_t n, int64_t lag, int64_t Ns, double* y,
+                                         cudaStream_t st, int64_t* launches);
 
 // Grassmann averages ----------------------------------------------------------------------------------
 enum GaMode : int {

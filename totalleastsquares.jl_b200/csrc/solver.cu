@@ -135,6 +135,9 @@ thread_local cudaMemPool_t t_pool = nullptr;
 // with min(M,N) > 512):
 // tlsq_rpca_f64 then repeats the solve on the dense device path (rpca_cb_host with the built-in hooks)
 thread_local bool t_dense_fallback = false;
+// set when a one-pass solve's rank estimate passed the kernel's cap and the streaming pipeline could not take over
+// (padded or in-place dual variable): lowrankfilter then repeats the solve on its materialising route
+thread_local bool t_fused_capped = false;
 
 struct DevBuf {                  // stream-ordered device allocation, freed on scope exit
     void* p = nullptr;
@@ -240,8 +243,9 @@ struct RpcaParams {
 struct RpcaOut {
     double* A = nullptr;  double* E = nullptr;  double* U = nullptr;  double* S = nullptr;  double* Vt = nullptr;
     int64_t* sv = nullptr;  int64_t* iters_done = nullptr;  int32_t* converged = nullptr;  double* hist = nullptr;
-    // lowrankfilter: anti-diagonal sums of the final (factored) A over this shard's Hankel rows [uh_r0, uh_r0 + M)
-    double* uh_sum = nullptr;  int64_t uh_r0 = 0;  int64_t uh_Ns = 0;
+    // lowrankfilter: sums of the final (factored) A over {(k, l): k lag + l = t} for this shard's Hankel rows
+    // [uh_r0, uh_r0 + M) and every sample t < uh_Ns; uh_lag is the embedding's lag
+    double* uh_sum = nullptr;  int64_t uh_r0 = 0;  int64_t uh_Ns = 0;  int64_t uh_lag = 1;
     // host-buffer entry points: pinned or pageable HOST destinations of A / E.  When set, their device->host copies are
     // issued on the side stream as soon as the output pass has produced them, i.e. they overlap the eigensolver and the
     // SVD refinement that still run on the main stream; *host_copied tells the caller that they were taken care of.
@@ -625,6 +629,7 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
         const int fused_cap = fused_max_rank(hankel);      // 16 for dense D, 32 for the implicit Hankel form
         if (fused && (svp > fused_cap || svpb[cur] > fused_cap)) {
             // rank estimate beyond the fused kernel: materialise W_k once and continue on the streaming pipeline
+            if (ldp != M || inplace_y || !all_legacy) t_fused_capped = true;
             if (ldp != M || inplace_y || !all_legacy)
                 return set_err(TLSQ_ERR_UNSUPPORTED, "rpca: rank estimate %d exceeds the one-pass kernel's cap of %d "
                                "(%s) and the streaming pipeline cannot take over (padded / in-place dual variable)", svp,
@@ -917,8 +922,8 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
         cudaStream_t ss = h->side;
         CK(cudaStreamWaitEvent(ss, h->ev_fork, 0));
         if (o.uh_sum)
-            CK(launch_unhankel_factors(Tb[last_idx], ldp, Vb[last_idx], svpb[last_idx], nonnegA, o.uh_r0, M, N, o.uh_Ns,
-                                       o.uh_sum, sms, ss, L));
+            CK(launch_unhankel_factors(Tb[last_idx], ldp, Vb[last_idx], svpb[last_idx], nonnegA, o.uh_r0, M, N, o.uh_lag,
+                                       o.uh_Ns, o.uh_sum, sms, ss, L));
         if (o.E || want_svd) {
             EpiArgs fe = {};
             fe.D = D; fe.Yp = Ybuf[prev_idx]; fe.Tp = Tb[prev_idx]; fe.Vp = Vb[prev_idx]; fe.svp_prev = svpb[prev_idx];
@@ -938,11 +943,12 @@ int rpca_core_once(tlsq_handle* h, MatSrc D, bool hankel, int64_t M, int64_t N, 
         }
     } else {
         if (o.uh_sum) {
-            // the rank estimate left the factored path: anti-diagonal sums from the dense A_k
+            // the rank estimate left the factored path: the unhankel sums from the dense A_k
             DevBuf bCnt;
             CK(bCnt.alloc((size_t)o.uh_Ns * 8, st));
             CK(cudaMemsetAsync(o.uh_sum, 0, (size_t)o.uh_Ns * 8, st));
-            CK(launch_unhankel_partial(Abuf[last_idx], o.uh_r0, M, N, 1, o.uh_Ns, o.uh_sum, bCnt.as<double>(), st, L));
+            CK(launch_unhankel_partial(Abuf[last_idx], o.uh_r0, M, N, o.uh_lag, o.uh_Ns, o.uh_sum, bCnt.as<double>(), st,
+                                       L));
         }
         // NB: E and W_k are recomputed from (A_{k-1}, Y_{k-1}); A_{k-1} may live in the caller's A buffer, so they must
         // be produced before A_k is copied there.
@@ -1223,8 +1229,10 @@ int lowrankfilter_dev(tlsq_handle* h, const double* y, int64_t Ns, int64_t n, in
     const int64_t K = (Ns - n) / lag + 1;                                                // :81
     if (!(p.lambda > 0.0)) p.lambda = 1.0 / sqrt((double)(K > n ? K : n));               // :157
     cudaStream_t st = h->stream;
-    // Factored unhankel (lag 1, tall enough for the factored iterate): A is never materialised -- the anti-diagonal
-    // sums are taken straight from A_k = clamp(T_k V_k'); sharded runs all-reduce the Ns partial sums.
+    // Factored unhankel (any lag, tall enough for the factored iterate): A is never materialised -- the unhankel sums
+    // are taken straight from A_k = clamp(T_k V_k'); sharded runs all-reduce the Ns partial sums.  Shards that neither
+    // the TMA SYRK nor the one-pass kernel can take (n != 256 with fewer than 4096 or an odd number of rows, n < 65)
+    // take the materialising routes below.
     {
         int64_t r0, Kl, per, Klast, r0last;
         shard_hankel_rows(K, h->nranks, h->rank, &r0, &Kl);
@@ -1233,26 +1241,53 @@ int lowrankfilter_dev(tlsq_handle* h, const double* y, int64_t Ns, int64_t n, in
         // the decision must be the same on every rank (collectives): test the regular shard and the last one
         auto shard_ok = [&](int64_t rows) {
             return rows >= 1 && (syrk_tma_eligible(reinterpret_cast<const double*>(uintptr_t(256)), rows, n, rows) ||
-                                 fused_eligible(MatSrc{y, 1}, true, rows, n));
+                                 fused_eligible(MatSrc{y, lag}, true, rows, n));
         };
-        if (lag == 1 && K >= n && n <= kEigMaxN && (h->nranks == 1 || shard_ok(per)) && shard_ok(Klast)) {
+        if (K >= n && n <= kEigMaxN && (h->nranks == 1 || shard_ok(per)) && shard_ok(Klast)) {
             CKR(check_rpca_args(Kl, n, p));
             DevBuf bSum;
             CK(bSum.alloc((size_t)Ns * 8, st));
             RpcaOut ol;
             ol.sv = sv; ol.iters_done = iters_done; ol.converged = converged; ol.hist = hist;
-            ol.uh_sum = bSum.as<double>(); ol.uh_r0 = r0; ol.uh_Ns = Ns;
-            MatSrc srcl{y + r0, 1};
-            CKR(rpca_core(h, srcl, true, Kl, n, p, ol));
-            CKR(allreduce(h, ol.uh_sum, (size_t)Ns, kNcclSum));
-            CK(launch_unhankel_divide_count(ol.uh_sum, K, n, Ns, yf, st, &h->launches));
-            CK(cudaStreamSynchronize(st));
-            return TLSQ_OK;
+            ol.uh_sum = bSum.as<double>(); ol.uh_r0 = r0; ol.uh_Ns = Ns; ol.uh_lag = lag;
+            MatSrc srcl{y + r0 * lag, lag};
+            t_dense_fallback = false;
+            t_fused_capped = false;
+            const int rc = rpca_core(h, srcl, true, Kl, n, p, ol);
+            if (rc == TLSQ_ERR_UNSUPPORTED && t_fused_capped) {
+                // rank estimate above the one-pass kernel's cap with no pipeline to hand over to (odd row count or Y
+                // in place): the same on every rank, as the pipeline choice is.  Repeat the solve on the materialising
+                // routes below, whose dense iterate has no rank cap at n <= 512.
+                t_fused_capped = false;
+                CK(cudaStreamSynchronize(st));
+            } else if (rc == TLSQ_ERR_UNSUPPORTED && t_dense_fallback && h->nranks == 1) {
+                // n > 512 and a rank estimate above 32: materialise the embedding, continue on the dense device path
+                t_dense_fallback = false;
+                CK(cudaStreamSynchronize(st));
+                DevBuf bA, bH;
+                CK(bA.alloc((size_t)K * n * 8, st));
+                CK(bH.alloc((size_t)K * n * 8, st));
+                CK(launch_hankel(y, K, n, lag, bH.as<double>(), st, &h->launches));
+                CKR(rpca_cb_host(h, bH.as<double>(), K, n, p, nullptr, nullptr, nullptr, bA.as<double>(), nullptr, nullptr,
+                                 nullptr, nullptr, sv, iters_done, converged, hist));
+                CK(launch_unhankel(bA.as<double>(), K, n, lag, Ns, yf, st, &h->launches));            // :127
+                CK(cudaStreamSynchronize(st));
+                return TLSQ_OK;
+            } else {
+                if (rc != TLSQ_OK) return rc;
+                CKR(allreduce(h, ol.uh_sum, (size_t)Ns, kNcclSum));
+                CK(launch_unhankel_divide_count(ol.uh_sum, K, n, lag, Ns, yf, st, &h->launches));
+                CK(cudaStreamSynchronize(st));
+                return TLSQ_OK;
+            }
         }
     }
     if (h->nranks > 1) {
-        // Row-sharded: every rank holds the (small) full signal and works on Hankel rows [r0, r1) through the same
-        // implicit index functor; only the n x n Gram, scalars and the anti-diagonal sums are all-reduced.
+        // Row-sharded, materialising each rank's K_local x n block of A: reached when a shard is not eligible for the
+        // factored route above (for example n = 300 with an odd row count in the last shard), when a one-pass solve there
+        // outgrew the kernel's rank cap, or with K < n.  Every rank holds the (small) full signal and works on Hankel rows
+        // [r0, r1) through the same implicit index functor; only the n x n Gram, scalars and the anti-diagonal sums are
+        // all-reduced.
         if (K < n || n > kEigMaxN)
             return set_err(TLSQ_ERR_UNSUPPORTED, "lowrankfilter (sharded): needs K >= n and n <= %d", kEigMaxN);
         const int64_t base = K / h->nranks, rem = K % h->nranks;
@@ -1276,6 +1311,8 @@ int lowrankfilter_dev(tlsq_handle* h, const double* y, int64_t Ns, int64_t n, in
         CK(cudaStreamSynchronize(st));
         return TLSQ_OK;
     }
+    // Single GPU, dense K x n A: K < n, a Hankel matrix neither the TMA SYRK nor the one-pass kernel takes, or a one-pass
+    // solve that outgrew the kernel's rank cap
     DevBuf bA, bH;
     CK(bA.alloc((size_t)K * n * 8, st));
     RpcaOut o;
